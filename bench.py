@@ -33,6 +33,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+CALLER_CWD = os.getcwd()  # where a relative --dump-outputs DIR is meant to be
 os.chdir(ROOT)  # scene files reference textures / sub-scenes relative to the CWD, like the reference CLI
 
 SCENE = "scenes/cornell-box-scene.json"
@@ -113,7 +114,7 @@ def host_threads() -> int:
 
 
 def oracle_sample(spp_sample: int, n_threads: int = 0, repeats: int = 1):
-    """Times the oracle on the bench workload at reduced spp.  Returns (Mrays/s, seconds, segments, threads)."""
+    """Times the oracle on the bench workload at reduced spp.  Returns (Mrays/s, seconds, segments, threads, image)."""
     if n_threads <= 0:
         n_threads = host_threads()
     from nr_ray_tracer_b200.scene_config import CameraConfig, load_scene
@@ -125,11 +126,30 @@ def oracle_sample(spp_sample: int, n_threads: int = 0, repeats: int = 1):
     best = None
     for _ in range(repeats):
         t0 = time.perf_counter()
-        _img, cnt = sc.render(cam, seed=0, n_threads=n_threads)
+        img, cnt = sc.render(cam, seed=0, n_threads=n_threads)
         dt = time.perf_counter() - t0
         if best is None or dt < best[1]:
             best = (cnt["segments"] / dt / 1e6, dt, cnt["segments"])
-    return best + (n_threads,)
+    return best + (n_threads, img)
+
+
+DUMP_BYTES = 64 * 1024 * 1024
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each array as out_dir/<name>.npy, at most DUMP_BYTES in all.  An array larger than its even share of what
+    the smaller ones leave is replaced by a fixed, seeded sample of its pixels (last axis kept; the same pixels for the
+    same shape), so that two builds run with the same arguments can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    left = DUMP_BYTES - 4096 * len(arrays)  # room for each .npy header
+    for k, (name, a) in enumerate(sorted(arrays.items(), key=lambda kv: kv[1].nbytes)):
+        share = left // (len(arrays) - k)
+        if a.nbytes > share:
+            px = a.reshape(-1, a.shape[-1])
+            keep = np.random.default_rng(0).choice(len(px), share // px[0].nbytes, replace=False)
+            a = px[np.sort(keep)]
+        left -= a.nbytes
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def run_reference(args):
@@ -142,9 +162,11 @@ def run_reference(args):
         oracle_sample(spp_sample)
     times, segs, threads = [], 0, 1
     for _ in range(args.steps):
-        _m, dt, s, threads = oracle_sample(spp_sample)
+        _m, dt, s, threads, img = oracle_sample(spp_sample)
         times.append(dt)
         segs += s
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"image": img, "segments": np.array([s], dtype=np.float64)})
     total = sum(times)
     value = segs / total / 1e6
     line = {
@@ -229,9 +251,11 @@ def run_b200(args):
             dist.barrier()
         torch.cuda.synchronize()
 
+    last = {}
+
     def step_device():
         """value: scene resident, result left on the device (rank 0 holds the assembled image)."""
-        _, st, _ = D.render_distributed(ctx, cam, rank, world, seed=0, mode=mode, gather=G)
+        last["image"], st, _ = D.render_distributed(ctx, cam, rank, world, seed=0, mode=mode, gather=G)
         return st
 
     def step_e2e(out_np=None):
@@ -308,11 +332,19 @@ def run_b200(args):
     my_segs = sum(s["segments"] for s in stats)
     mode_used = stats[0]["mode"]
     kernel_name = KERNEL.get(mode_used, "?")
+    # ---- untimed: what the last timed step of each path handed its caller (the gather buffers are reused below)
+    outputs = {}
+    if args.dump_outputs:
+        outputs["segments"] = np.array([total(stats[-1:], "segments")], dtype=np.float64)
+        if rank == 0:
+            outputs["image"] = last["image"].cpu().numpy()
 
     # ---- timed: end to end through the public API (host buffers)
     pinned_np = pinned.numpy() if rank == 0 else None
     step_e2e(pinned_np)
     ms_e2e, stats_e2e = timed(lambda: step_e2e(pinned_np), args.steps)
+    if args.dump_outputs and rank == 0:
+        outputs["e2e_image"] = pinned_np.copy()
     segs_e2e = total(stats_e2e, "segments")
     e2e_value = segs_e2e / (sum(ms_e2e) * 1e-3) / 1e6
     e2e_pageable = None
@@ -395,7 +427,7 @@ def run_b200(args):
         # ---- CPU baseline on a bounded sample (rank 0, N=1 only)
         cpu = None
         if world == 1 and not args.no_cpu:
-            m, dt, s, threads = oracle_sample(args.cpu_spp)
+            m, dt, s, threads, _ = oracle_sample(args.cpu_spp)
             cpu = {"value": m, "unit": UNIT, "cores": threads, "kind": "port",
                    "sample": f"{SCENE} {args.width}x{args.height} depth {DEPTH} at {args.cpu_spp} spp "
                              f"({s} segments in {dt:.1f} s; C++ restatement of the reference algorithm, OpenMP)"}
@@ -426,6 +458,8 @@ def run_b200(args):
         }
         if identical is not None:
             line["multi_gpu_image_identical_to_single_gpu"] = identical
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
@@ -455,7 +489,14 @@ def main():
     ap.add_argument("--cpu-spp", type=int, default=128, help="spp of the bounded cpu_baseline sample")
     ap.add_argument("--ref-spp", type=int, default=32, help="spp per step of the --impl reference arm")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (f32 image, f64 "
+                         "segment count; at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs:
+        args.dump_outputs = os.path.join(CALLER_CWD, args.dump_outputs)
     SCENE, WIDTH, HEIGHT, SPP, DEPTH = args.scene, args.width, args.height, args.spp, args.depth
     if args.impl == "reference":
         return run_reference(args)
