@@ -488,6 +488,40 @@ uint32_t nrrt_chunk_starts(uint32_t samples_per_pixel, uint64_t total_pixels, ui
 uint32_t nrrt_work_items(uint32_t width, uint32_t height, uint32_t samples_per_pixel, uint32_t rank, uint32_t world,
                          uint32_t rows_per_block, uint32_t first, uint32_t n, uint32_t* out);
 
+/* The same for one pass of a progressive render: the work items of chunks [c0, c1) (c1 clamped to n_chunks), numbered
+ * from 0 in the order that pass hands them out.  nrrt_work_items is c0 = 0, c1 = all.  Returns 0 also when c0 > n_chunks. */
+uint32_t nrrt_pass_items(uint32_t width, uint32_t height, uint32_t samples_per_pixel, uint32_t rank, uint32_t world,
+                         uint32_t rows_per_block, uint32_t c0, uint32_t c1, uint32_t first, uint32_t n, uint32_t* out);
+
+/* ---- progressive rendering ---------------------------------------------------------------------------------------
+ * One frame rendered in passes on one context.  A pass renders the next whole chunks of every owned pixel (pass
+ * boundaries are nrrt_chunk_starts boundaries) and adds their partial sums, in chunk order, into a per-pixel f64 sum the
+ * handle keeps in device memory (24 B per owned pixel, owned rows packed: row j, column x, RGB).  A pixel's sample s
+ * traces the same path in whichever pass it runs, so:
+ *   - after the last pass the image is nrrt_render's, bit for bit, whatever the passes were;
+ *   - after samples [0, s) the image is the sum over those chunks divided by s (the CPU oracle's render_chunked);
+ *   - a pass needs scratch for its own chunks only (24 B per owned pixel and chunk).
+ * camera->samples_per_pixel, opts->seed / mode / rank / world / rows_per_block / max_slots are fixed at creation; the
+ * output flags of opts are ignored (nrrt_accum_image takes them), NRRT_RENDER_COUNT is honoured.  Every call fails with
+ * NRRT_ERR_NO_SCENE once nrrt_scene_upload has replaced the context's scene.  Error messages: nrrt_last_error(ctx).
+ * Free the handle before its context. */
+typedef struct nrrt_accum nrrt_accum;
+int nrrt_accum_create(nrrt_ctx* ctx, const nrrt_camera* camera, const nrrt_render_opts* opts, nrrt_accum** out);
+/* Renders the next whole chunks until at least min(min_samples, spp) samples per pixel are done (nothing if they are
+ * already; stats are then zero but for pixels).  stats (may be NULL) describe this pass. */
+int nrrt_accum_render(nrrt_accum* accum, uint32_t min_samples, nrrt_render_stats* stats);
+/* Samples per pixel done so far (a chunk boundary; spp when the frame is complete). */
+uint32_t nrrt_accum_samples(const nrrt_accum* accum);
+/* The image so far: sums / samples done, as f32, laid out as nrrt_render lays out out_rgb (flags
+ * NRRT_RENDER_OUT_DEVICE / NRRT_RENDER_OUT_PACKED as there).  NRRT_ERR_INVALID before the first pass. */
+int nrrt_accum_image(nrrt_accum* accum, float* out_rgb, uint32_t flags);
+/* Host copy of the sums (stats.pixels x 3 f64, owned rows packed) and the samples they hold, e.g. to resume later. */
+int nrrt_accum_save(const nrrt_accum* accum, double* sums, uint32_t* samples_done);
+/* Loads what nrrt_accum_save wrote, into an accumulator of the same frame (camera, opts, scene), possibly on another
+ * context.  NRRT_ERR_INVALID if samples_done is not a chunk boundary of the frame (so also above spp). */
+int nrrt_accum_restore(nrrt_accum* accum, const double* sums, uint32_t samples_done);
+void nrrt_accum_free(nrrt_accum* accum);
+
 /* sizeof() of the ABI structs as compiled (which = 0..18: object, material, texture,
  * image, graph_desc, camera_config, camera, node, box, xform, instance, scene_desc, hit, trace_stats,
  * render_opts, render_stats, camera_file, wnode, hit_compact) so a binding can verify its mirror of this header. */

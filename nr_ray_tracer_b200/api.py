@@ -76,6 +76,16 @@ def lib() -> C.CDLL:
         L.nrrt_chunk_starts.argtypes = [C.c_uint32, C.c_uint64, C.POINTER(C.c_uint32), C.c_uint32]
         L.nrrt_work_items.restype = C.c_uint32
         L.nrrt_work_items.argtypes = [C.c_uint32] * 8 + [C.POINTER(C.c_uint32)]
+        L.nrrt_pass_items.restype = C.c_uint32
+        L.nrrt_pass_items.argtypes = [C.c_uint32] * 10 + [C.POINTER(C.c_uint32)]
+        L.nrrt_accum_create.argtypes = [C.c_void_p, C.POINTER(A.Camera), C.POINTER(A.RenderOpts), C.POINTER(C.c_void_p)]
+        L.nrrt_accum_render.argtypes = [C.c_void_p, C.c_uint32, C.POINTER(A.RenderStats)]
+        L.nrrt_accum_samples.restype = C.c_uint32
+        L.nrrt_accum_samples.argtypes = [C.c_void_p]
+        L.nrrt_accum_image.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32]
+        L.nrrt_accum_save.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(C.c_uint32)]
+        L.nrrt_accum_restore.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32]
+        L.nrrt_accum_free.argtypes = [C.c_void_p]
         L.nrrt_abi_sizeof.restype = C.c_size_t
         L.nrrt_abi_sizeof.argtypes = [C.c_int]
         _lib = L
@@ -104,6 +114,28 @@ def work_items(width: int, height: int, samples_per_pixel: int, rank: int = 0, w
         lib().nrrt_work_items(width, height, samples_per_pixel, rank, world, rows_per_block, 0, n,
                               out.ctypes.data_as(C.POINTER(C.c_uint32)))
     return out
+
+
+def pass_items(width: int, height: int, samples_per_pixel: int, c0: int, c1: int, rank: int = 0, world: int = 1,
+               rows_per_block: int = 8) -> np.ndarray:
+    """The work items of one progressive pass over chunks [c0, c1) in hand-out order, (n_items, 4) uint32 as in
+    work_items (nrrt_pass_items: the kernels' decode with the pass's chunk offset, run on the host)."""
+    args = (width, height, samples_per_pixel, rank, world, rows_per_block, c0, c1)
+    n = lib().nrrt_pass_items(*args, 0, 0, None)
+    out = np.zeros((n, 4), dtype=np.uint32)
+    if n:
+        lib().nrrt_pass_items(*args, 0, n, out.ctypes.data_as(C.POINTER(C.c_uint32)))
+    return out
+
+
+def owned_rows(height: int, rank: int = 0, world: int = 1, rows_per_block: int = 0) -> int:
+    """Rows rank `rank` of `world` renders: row-blocks b with b % world == rank (rows_per_block 0 -> 8)."""
+    R = rows_per_block or 8
+    return sum(min(R, height - b * R) for b in range(rank, (height + R - 1) // R, world))
+
+
+_STATS = ("paths", "segments", "launches", "device_ms", "extend_ms", "extend_launches", "pixels", "mode", "node_visits",
+          "box_exact", "prim_tests", "inst_entries", "inst_misses")
 
 
 def camera_build(cfg: A.CameraConfig) -> A.Camera:
@@ -297,10 +329,14 @@ class Context:
             ptr = C.c_void_p(out.ctypes.data)
         self._check(lib().nrrt_render(self._h, C.byref(cam), C.byref(opts), ptr, C.cast(cb, C.c_void_p) if cb else None,
                                       None, C.byref(st)))
-        stats = {k: getattr(st, k) for k in ("paths", "segments", "launches", "device_ms", "extend_ms",
-                                             "extend_launches", "pixels", "mode", "node_visits", "box_exact",
-                                             "prim_tests", "inst_entries", "inst_misses")}
+        stats = {k: getattr(st, k) for k in _STATS}
         return (None if out_device_ptr is not None else out), stats
+
+    def progressive(self, cam: A.Camera, seed: int = 0, mode: int = A.MODE_AUTO, rank: int = 0, world: int = 1,
+                    rows_per_block: int = 0, max_slots: int = 0) -> "Progressive":
+        """One frame of `cam` rendered in passes (nrrt_accum_*): see Progressive."""
+        return Progressive(self, cam, seed=seed, mode=mode, rank=rank, world=world, rows_per_block=rows_per_block,
+                           max_slots=max_slots)
 
 
     def encode_rgb8(self, image: Optional[np.ndarray] = None, gamma: float = 0.5, device_ptr: Optional[int] = None,
@@ -316,6 +352,85 @@ class Context:
         out = np.zeros((h, w, 3), dtype=np.uint8)
         self._check(lib().nrrt_encode_rgb8(self._h, ptr, w, h, gamma, flags, C.c_void_p(out.ctypes.data)))
         return out
+
+
+class Progressive:
+    """A frame rendered in passes of whole work chunks, summed on the GPU into per-pixel f64 sums (nrrt_accum_*).
+
+    render(min_samples) renders the next chunks until at least that many samples per pixel are done (pass boundaries
+    are chunk_starts() boundaries); image() is the frame so far, sums / samples.  The finished frame is
+    Context.render's image bit for bit, whatever the passes.  state() / restore() save and resume the sums.
+    Keeps its Context alive; the scene must stay the one uploaded when the frame was created."""
+
+    def __init__(self, ctx: Context, cam: A.Camera, seed: int = 0, mode: int = A.MODE_AUTO, rank: int = 0,
+                 world: int = 1, rows_per_block: int = 0, max_slots: int = 0):
+        self.ctx = ctx
+        self.camera = cam
+        self.samples_per_pixel = max(1, cam.samples_per_pixel)
+        self.rows = owned_rows(cam.height, rank, world, rows_per_block)
+        opts = A.RenderOpts(seed=seed, mode=mode, rank=rank, world=world, rows_per_block=rows_per_block,
+                            max_slots=max_slots, flags=0)
+        h = C.c_void_p()
+        ctx._check(lib().nrrt_accum_create(ctx._h, C.byref(cam), C.byref(opts), C.byref(h)))
+        self._h = h
+
+    def close(self):
+        if getattr(self, "_h", None):
+            lib().nrrt_accum_free(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    @property
+    def samples(self) -> int:
+        """Samples per pixel done so far."""
+        return int(lib().nrrt_accum_samples(self._h))
+
+    def render(self, min_samples: int) -> dict:
+        """One pass: the next whole chunks until at least min(min_samples, spp) samples are done.  Returns its stats."""
+        st = A.RenderStats()
+        self.ctx._check(lib().nrrt_accum_render(self._h, min(int(min_samples), self.samples_per_pixel), C.byref(st)))
+        return {k: getattr(st, k) for k in _STATS}
+
+    def image(self, out: Optional[np.ndarray] = None, packed: bool = False,
+              out_device_ptr: Optional[int] = None) -> Optional[np.ndarray]:
+        """The frame so far as linear f32 RGB, laid out as Context.render lays it out (full image with this rank's rows
+        written, or packed=True: this rank's rows only).  None for device output."""
+        flags = (A.RENDER_OUT_DEVICE if out_device_ptr is not None else 0) | (A.RENDER_OUT_PACKED if packed else 0)
+        if out_device_ptr is not None:
+            ptr = C.c_void_p(out_device_ptr)
+        else:
+            if out is None:
+                out = np.zeros((self.rows if packed else self.camera.height, self.camera.width, 3), dtype=np.float32)
+            assert out.dtype == np.float32 and out.flags.c_contiguous
+            assert out.size == (self.rows if packed else self.camera.height) * self.camera.width * 3
+            ptr = C.c_void_p(out.ctypes.data)
+        self.ctx._check(lib().nrrt_accum_image(self._h, ptr, flags))
+        return None if out_device_ptr is not None else out
+
+    def state(self):
+        """(samples done, f64 sums (owned rows, W, 3) in owned-row order): what restore() takes."""
+        sums = np.zeros((self.rows, self.camera.width, 3), dtype=np.float64)
+        n = C.c_uint32()
+        self.ctx._check(lib().nrrt_accum_save(self._h, C.c_void_p(sums.ctypes.data), C.byref(n)))
+        return int(n.value), sums
+
+    def restore(self, samples: int, sums: np.ndarray):
+        """Resumes from state(): `samples` must be a chunk boundary of this frame."""
+        sums = np.ascontiguousarray(sums, dtype=np.float64)
+        if sums.size != self.rows * self.camera.width * 3:
+            raise ValueError(f"sums must hold {self.rows} x {self.camera.width} x 3 values")
+        self.ctx._check(lib().nrrt_accum_restore(self._h, C.c_void_p(sums.ctypes.data), int(samples)))
 
 
 def render_multi(devices, host_scene: "HostScene", cam: A.Camera, out: Optional[np.ndarray] = None, seed: int = 0,
@@ -362,3 +477,15 @@ class Scene:
         """Scene::render -> linear f32 RGB image (H, W, 3), no gamma, no clamp."""
         img, self.last_stats = self.ctx.render(self.camera, progress=progress, **kw)
         return img
+
+    def render_progressive(self, every: Optional[int] = None, **kw):
+        """Scene::render in passes: yields (samples done, image so far) after each pass.  every=None: one pass per work
+        chunk; every=N: passes up to the next multiple of N samples (rounded up to a chunk boundary).  The last image
+        yielded is render()'s.  kw: Context.progressive's options (seed, mode, ...)."""
+        if every is not None and every < 1:
+            raise ValueError("every must be >= 1")
+        with self.ctx.progressive(self.camera, **kw) as p:
+            while p.samples < p.samples_per_pixel:
+                done = p.samples
+                self.last_stats = p.render(done + 1 if every is None else (done // every + 1) * every)
+                yield p.samples, p.image()

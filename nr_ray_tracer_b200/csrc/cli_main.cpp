@@ -5,8 +5,10 @@
 //   ->  build  ->  scene.render()  ->  gamma_correction(gamma)  ->  to_rgb8  ->  encode by extension
 // Flags and NR_RT_CAMERA_* environment fallbacks follow ray-tracer/src/cli.rs:113-270 (field of view and defocus
 // angle in degrees; image size needs exactly two of width / height / aspect ratio; default output out.png,
-// default gamma 0.5).  Additions: --seed, --mode auto|pool|fused|wavefront|megakernel, --device N, --gpus N.
+// default gamma 0.5).  Additions: --seed, --mode auto|pool|fused|wavefront|megakernel, --device N, --gpus N,
+// --preview-every N.
 // Encoders available without external libraries: .png (stored/uncompressed deflate) and .ppm.
+#include <algorithm>
 #include <cerrno>
 #include <chrono>
 #include <cstdint>
@@ -110,6 +112,24 @@ static void write_ppm(FILE* f, const uint8_t* rgb, uint32_t w, uint32_t h) {
     std::fprintf(f, "P6\n%u %u\n255\n", w, h);
     std::fwrite(rgb, 1, (size_t)w * h * 3, f);
 }
+static void write_image(FILE* f, bool png, const uint8_t* rgb, uint32_t w, uint32_t h) {
+    if (png) write_png(f, rgb, w, h);
+    else write_ppm(f, rgb, w, h);
+}
+// Replaces `path` by a complete image: written to a temporary file next to it, then renamed over it, so that a viewer
+// watching a progressive render never reads a half-written file.
+static void replace_image(const std::string& path, bool png, const uint8_t* rgb, uint32_t w, uint32_t h) {
+    const std::string tmp = path + ".tmp" + std::to_string((long)getpid());
+    FILE* f = std::fopen(tmp.c_str(), "wb");
+    if (!f) die("cannot open " + tmp + ": " + std::strerror(errno));
+    write_image(f, png, rgb, w, h);
+    const bool ok = std::fflush(f) == 0 && !std::ferror(f);
+    if (std::fclose(f) != 0 || !ok || std::rename(tmp.c_str(), path.c_str()) != 0) {
+        const std::string why = std::strerror(errno);
+        std::remove(tmp.c_str());
+        die("cannot write " + path + ": " + why);
+    }
+}
 
 // Unsigned decimal integer, whole string, no sign, <= max (clap rejects "-1", "1e3", "" and overflow alike).
 static bool parse_u64(const char* s, uint64_t max, uint64_t* out) {
@@ -140,6 +160,9 @@ static void usage() {
         "      --gpus <N>                 render on GPUs device .. device+N-1 of this box (rows interleaved across them,\n"
         "                                 same image bit for bit; env NR_RT_GPUS)\n"
         "      --bvh reference|sah   reference = the reference's BVH (default), sah = surface-area-heuristic inner nodes\n"
+        "      --preview-every <N>        render in passes and rewrite the output file whenever another N samples per\n"
+        "                                 pixel are done (passes end on whole work chunks; the final image is the same;\n"
+        "                                 one GPU only)\n"
         "  -v, --verbose                  print timing\n"
         "Every camera option falls back to NR_RT_CAMERA_<NAME> (e.g. NR_RT_CAMERA_SAMPLES_PER_PIXEL).");
 }
@@ -183,7 +206,7 @@ int main(int argc, char** argv) {
     std::string scene_path, output = "out.png", mode = "auto", bvh = "reference";
     bool force = false, verbose = false;
     float gamma = 0.5f;  // constants.rs:1
-    uint64_t seed = 0;
+    uint64_t seed = 0, preview_every = 0;
     int device = 0, gpus = 1;
     if (const char* e = std::getenv("NR_RT_GPUS")) {
         uint64_t x = 0;
@@ -276,6 +299,10 @@ int main(int argc, char** argv) {
             uint64_t x = 0;
             if (!parse_u64(v, 64, &x) || x == 0) die("invalid value '" + std::string(v) + "' for --gpus");
             gpus = (int)x;
+        } else if (a == "--preview-every") {
+            const char* v = need();
+            if (!parse_u64(v, 0xFFFFFFFFull, &preview_every) || preview_every == 0)
+                die("invalid value '" + std::string(v) + "' for --preview-every");
         }
         else if (a == "-W") { if (!set_camera("width", need())) die("invalid width"); }
         else if (a == "-H") { if (!set_camera("height", need())) die("invalid height"); }
@@ -290,6 +317,8 @@ int main(int argc, char** argv) {
         else die("unexpected argument '" + a + "'");
     }
     if (scene_path.empty()) die("missing <SCENE>");
+    if (preview_every && gpus > 1)
+        die("--preview-every renders on one GPU: it cannot be combined with --gpus " + std::to_string(gpus));
     auto ends = [&](const char* suf) {
         size_t n = std::strlen(suf);
         return output.size() >= n && output.compare(output.size() - n, n, suf) == 0;
@@ -344,14 +373,45 @@ int main(int argc, char** argv) {
         if (nrrt_render_multi(devs.data(), gpus, nrrt_host_scene_desc(hs), &cam, &opts, image.data(),
                               verbose ? on_progress : nullptr, nullptr, &st, msg, sizeof msg) != NRRT_OK)
             die(msg);
+    } else if (preview_every) {
+        // progressive: each pass renders up to the next multiple of N samples (rounded up to a chunk boundary), then the
+        // image so far replaces the output file; the last pass completes the frame, which is nrrt_render's bit for bit
+        std::fclose(out);  // (opened above only for the create-new check: every image goes through replace_image)
+        out = nullptr;
+        nrrt_accum* acc = nullptr;
+        if (nrrt_accum_create(ctx, &cam, &opts, &acc) != NRRT_OK) die(nrrt_last_error(ctx));
+        const uint32_t spp = cam.samples_per_pixel ? cam.samples_per_pixel : 1;
+        std::vector<uint8_t> preview(image.size());
+        std::memset(&st, 0, sizeof st);
+        while (nrrt_accum_samples(acc) < spp) {
+            const uint64_t target = (nrrt_accum_samples(acc) / preview_every + 1) * preview_every;
+            nrrt_render_stats ps;
+            if (nrrt_accum_render(acc, (uint32_t)std::min<uint64_t>(target, spp), &ps) != NRRT_OK) die(nrrt_last_error(ctx));
+            st.paths += ps.paths, st.segments += ps.segments, st.launches += ps.launches, st.device_ms += ps.device_ms;
+            const uint32_t done = nrrt_accum_samples(acc);
+            if (verbose)
+                std::fprintf(stderr, "pass: %u / %u samples  (%.3f s)\n", done, spp,
+                             std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count());
+            if (done < spp) {
+                if (nrrt_accum_image(acc, image.data(), 0) != NRRT_OK ||
+                    nrrt_encode_rgb8(ctx, image.data(), cam.width, cam.height, gamma, 0, preview.data()) != NRRT_OK)
+                    die(nrrt_last_error(ctx));
+                replace_image(output, png, preview.data(), cam.width, cam.height);
+            }
+        }
+        if (nrrt_accum_image(acc, image.data(), 0) != NRRT_OK) die(nrrt_last_error(ctx));
+        nrrt_accum_free(acc);
     } else if (nrrt_render(ctx, &cam, &opts, image.data(), verbose ? on_progress : nullptr, nullptr, &st) != NRRT_OK)
         die(nrrt_last_error(ctx));
     auto t1 = std::chrono::steady_clock::now();
     std::vector<uint8_t> rgb8(image.size());
     if (nrrt_encode_rgb8(ctx, image.data(), cam.width, cam.height, gamma, 0, rgb8.data()) != NRRT_OK) die(nrrt_last_error(ctx));
-    if (png) write_png(out, rgb8.data(), cam.width, cam.height);
-    else write_ppm(out, rgb8.data(), cam.width, cam.height);
-    std::fclose(out);
+    if (out) {
+        write_image(out, png, rgb8.data(), cam.width, cam.height);
+        std::fclose(out);
+    } else {
+        replace_image(output, png, rgb8.data(), cam.width, cam.height);
+    }
     if (verbose) {
         double s = std::chrono::duration<double>(t1 - t0).count();
         std::printf("Rendering: done in %.3f secs  (%ux%u, %u spp, depth %u; %llu paths, %llu ray segments, %.1f Mrays/s)\n",

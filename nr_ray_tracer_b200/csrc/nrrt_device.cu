@@ -77,7 +77,9 @@ struct RenderParams {
     uint32_t chunk;          // samples of an equal-size work item (the first n_eq chunks of a pixel)
     uint32_t n_eq;           // equal chunks; they cover samples [0, n_eq * chunk)
     uint32_t n_chunks;       // work items per pixel = n_eq + the halving chunks over the remaining samples
-    uint32_t n_items;        // n_owned_pixels * n_chunks
+    uint32_t c0;             // first chunk of this launch: it renders chunks [c0, c0 + n_items / n_owned_pixels)
+    uint32_t n_items;        // n_owned_pixels * (chunks of this launch); items and partials are numbered from c0
+    uint32_t long_end;       // item where this launch's equal chunks end (item_block_size)
     uint32_t n_slots;        // paths in flight
     uint32_t n_warps;        // warps that fetch work-item blocks (persistent kernels)
     uint32_t rank, world, rows_per_block;
@@ -114,13 +116,12 @@ __host__ __device__ __forceinline__ void owned_pixel(const nrrt_camera& cam, con
 // Size of the next block of work items a warp takes: NRRT_ITEM_BLOCK while work is plentiful, shrinking to 32 (one per
 // lane) as the image runs out — so that the render does not end with a few warps still holding four items per lane
 // (a 400x225 image is 9 ms of work: blocks of 128 to the end cost it 20 %).  `next` is the global counter as last seen.
-// Items are chunk-major and the equal chunks come first: the LONG items end at item n_eq * n_owned_pixels, and a warp
+// Items are chunk-major and the equal chunks come first: the LONG items end at item long_end, and a warp
 // that has just taken 128 of them when they run out keeps the GPU waiting for 4 long items per lane while everyone
 // else is through the short tail chunks — so the blocks also shrink towards that point (measured at N = 8, where a
 // GPU has 130 ms of work: 7 ms lost without this).
 __device__ __forceinline__ uint32_t item_block_size(const RenderParams& P, unsigned long long next, uint32_t need) {
-    const uint32_t long_end = P.n_eq * P.n_owned_pixels;  // (fits: n_items does)
-    const uint32_t end = next < long_end ? long_end : P.n_items;
+    const uint32_t end = next < P.long_end ? P.long_end : P.n_items;
     const uint32_t left = next < end ? end - (uint32_t)next : 0u;
     uint32_t b = left / (2u * max(P.n_warps, 1u));
     b = min(max(b, 32u), (uint32_t)NRRT_ITEM_BLOCK);
@@ -131,10 +132,12 @@ struct WorkItem {
     uint32_t x, y;        // pixel
     uint32_t sample_end;  // one past the last sample of the chunk
 };
-// item -> pixel + sample range; returns the first sample
+// item -> pixel + sample range; returns the first sample.  The chunk c is absolute (the launch's item 0 is chunk c0's
+// first pixel), so a pixel's samples and their Philox counters do not depend on which launch renders them.
 __host__ __device__ __forceinline__ uint32_t decode_item(const nrrt_camera& cam, const RenderParams& P, uint32_t item,
                                                          WorkItem& wi) {
     uint32_t c = P.div_pixels.div(item), po = item - c * P.n_owned_pixels;
+    c += P.c0;
     uint32_t j;
     owned_pixel(cam, P, po, wi.x, wi.y, j);
     const uint32_t spp = cam.samples_per_pixel;
@@ -320,20 +323,27 @@ k_render_mega(const __grid_constant__ DevScene S, const __grid_constant__ nrrt_c
     }
 }
 
-// per-pixel sample accumulation: add the chunk partials in chunk order, divide by spp, cast to f32
-// (camera.rs:329-337)
+// per-pixel sample accumulation: add the launch's n_items / n_owned_pixels chunk partials in chunk order, divide by
+// the samples summed, cast to f32 (camera.rs:329-337).  acc (may be null: start from zero) is the pixel's running f64
+// sum over earlier chunks, in owned-row order (j, x), and receives the new sum; out (may be null) the image.  A render
+// in passes thus makes the one-shot render's additions, in the same order.
 __global__ void k_resolve(const __grid_constant__ nrrt_camera cam, const __grid_constant__ RenderParams P,
-                          const double* __restrict__ partials, float* __restrict__ out, bool packed) {
+                          const double* __restrict__ partials, double* __restrict__ acc, double samples,
+                          float* __restrict__ out, bool packed) {
     uint32_t po = blockIdx.x * blockDim.x + threadIdx.x;
     if (po >= P.n_owned_pixels) return;
-    d3 s = mk3(0.0, 0.0, 0.0);
-    for (uint32_t c = 0; c < P.n_chunks; ++c) {
+    uint32_t x, y, j;
+    owned_pixel(cam, P, po, x, y, j);
+    const size_t ab = ((size_t)j * cam.width + x) * 3;
+    d3 s = acc ? mk3(acc[ab], acc[ab + 1], acc[ab + 2]) : mk3(0.0, 0.0, 0.0);
+    const uint32_t n_chunks = P.n_items / P.n_owned_pixels;
+    for (uint32_t c = 0; c < n_chunks; ++c) {
         size_t b = ((size_t)c * P.n_owned_pixels + po) * 3;
         s = add3(s, mk3(partials[b], partials[b + 1], partials[b + 2]));
     }
-    d3 col = div3(s, (double)cam.samples_per_pixel);
-    uint32_t x, y, j;
-    owned_pixel(cam, P, po, x, y, j);
+    if (acc && n_chunks) acc[ab] = s.x, acc[ab + 1] = s.y, acc[ab + 2] = s.z;
+    if (!out) return;
+    d3 col = div3(s, samples);
     size_t ob = ((size_t)(packed ? j : y) * cam.width + x) * 3;  // packed: the rank's rows in ascending order
     out[ob] = (float)col.x, out[ob + 1] = (float)col.y, out[ob + 2] = (float)col.z;
 }
@@ -861,6 +871,7 @@ struct nrrt_ctx {
     cudaStream_t side = nullptr;       // progress polling while a single-launch render runs (created on first use)
     void* enc_buf = nullptr;           // output-stage scratch (nrrt_encode_rgb8), grown on demand
     size_t enc_bytes = 0;
+    uint64_t scene_gen = 0;            // bumped by every nrrt_scene_upload: an nrrt_accum belongs to one scene
 };
 
 #define CK(call)                                                                                   \
@@ -1159,6 +1170,7 @@ int nrrt_scene_upload(nrrt_ctx* ctx, const nrrt_scene_desc* sc) {
     CK(cudaSetDevice(ctx->device));
     CK(cudaStreamSynchronize(ctx->stream));
     free_scene(ctx);
+    ++ctx->scene_gen;
     DevScene D{};
     int rc;
 #define UP(field, host, count)                                          \
@@ -1613,9 +1625,10 @@ static uint32_t owned_rows(uint32_t H, uint32_t rank, uint32_t world, uint32_t R
 }
 
 // Partition and work-item fields of RenderParams (everything decode_item / owned_pixel / item_block_size read, bar the
-// slot counts): shared by nrrt_render and nrrt_work_items.  Returns nullptr or the reason it cannot be done.
+// slot counts) of a launch over chunks [c0, c1) (c1 clamped to the pixel's chunks): shared by the renders and
+// nrrt_work_items / nrrt_pass_items.  Returns nullptr or the reason it cannot be done.
 static const char* work_item_params(RenderParams& P, uint32_t W, uint32_t H, uint32_t spp, uint32_t rank, uint32_t world,
-                                    uint32_t rows_per_block) {
+                                    uint32_t rows_per_block, uint32_t c0 = 0, uint32_t c1 = 0xFFFFFFFFu) {
     const uint64_t total_pixels = (uint64_t)W * H;
     P.rank = rank, P.world = world, P.rows_per_block = rows_per_block;
     P.n_owned_pixels = owned_rows(H, rank, world, rows_per_block) * W;
@@ -1639,9 +1652,13 @@ static const char* work_item_params(RenderParams& P, uint32_t W, uint32_t H, uin
     //    up to 2.1 Mpixel, 8 at 4K (1080p x 1024 spp: 27 x 37 + 25; 4K x 4096 spp: 8 items per pixel, 1.6 GB where
     //    round 1 needed 6.4 GB).
     chunk_schedule(spp, total_pixels, P.chunk, P.n_eq, P.n_chunks);
-    const uint64_t n_items64 = (uint64_t)P.n_owned_pixels * P.n_chunks;
+    c1 = std::min(c1, P.n_chunks);
+    if (c0 > c1) return "chunk range past the last chunk";
+    const uint64_t n_items64 = (uint64_t)P.n_owned_pixels * (c1 - c0);
     if (n_items64 > 0xFFFFFFF0ull) return "too many work items";
+    P.c0 = c0;
     P.n_items = (uint32_t)n_items64;
+    P.long_end = (std::min(std::max(P.n_eq, c0), c1) - c0) * P.n_owned_pixels;  // (fits: n_items does)
     P.n_slots = P.n_warps = 0;
     P.div_pixels = FastDiv::make(P.n_owned_pixels);
     P.div_rows = FastDiv::make(rows_per_block);
@@ -1666,11 +1683,11 @@ static const char* work_item_params(RenderParams& P, uint32_t W, uint32_t H, uin
     return nullptr;
 }
 
-// Work items [first, first + n) of one rank's render, decoded by the very functions the kernels use: 4 values per item
-// (x, y, first sample, one past the last sample).  Returns the number of items of that render, 0 if the arguments are
-// not ones nrrt_render would take.
-uint32_t nrrt_work_items(uint32_t width, uint32_t height, uint32_t samples_per_pixel, uint32_t rank, uint32_t world,
-                         uint32_t rows_per_block, uint32_t first, uint32_t n, uint32_t* out) {
+// Work items [first, first + n) of one rank's launch over chunks [c0, c1), decoded by the very functions the kernels
+// use: 4 values per item (x, y, first sample, one past the last sample).  Returns the number of items of that launch, 0
+// if the arguments are not ones the renders would take.
+uint32_t nrrt_pass_items(uint32_t width, uint32_t height, uint32_t samples_per_pixel, uint32_t rank, uint32_t world,
+                         uint32_t rows_per_block, uint32_t c0, uint32_t c1, uint32_t first, uint32_t n, uint32_t* out) {
     if (width == 0 || height == 0 || (uint64_t)width * height > 0x7FFFFFFFull) return 0;
     if (world == 0) world = 1;
     if (rank >= world) return 0;
@@ -1680,7 +1697,7 @@ uint32_t nrrt_work_items(uint32_t width, uint32_t height, uint32_t samples_per_p
     nrrt_camera cam;
     std::memset(&cam, 0, sizeof cam);
     cam.width = width, cam.height = height, cam.samples_per_pixel = std::max<uint32_t>(samples_per_pixel, 1);
-    if (work_item_params(P, width, height, cam.samples_per_pixel, rank, world, rows_per_block)) return 0;
+    if (work_item_params(P, width, height, cam.samples_per_pixel, rank, world, rows_per_block, c0, c1)) return 0;
     for (uint32_t i = 0; out && i < n && (uint64_t)first + i < P.n_items; ++i) {
         WorkItem wi;
         const uint32_t s0 = decode_item(cam, P, first + i, wi);
@@ -1689,49 +1706,29 @@ uint32_t nrrt_work_items(uint32_t width, uint32_t height, uint32_t samples_per_p
     return P.n_items;
 }
 
-int nrrt_render(nrrt_ctx* ctx, const nrrt_camera* cam, const nrrt_render_opts* opts_in, float* out_rgb,
-                nrrt_progress_fn progress, void* user, nrrt_render_stats* stats) {
-    if (!ctx) return NRRT_ERR_INVALID;
-    if (!ctx->has_scene) {
-        ctx->err = "nrrt_render before nrrt_scene_upload";
-        return NRRT_ERR_NO_SCENE;
-    }
-    if (!cam || !out_rgb || cam->width == 0 || cam->height == 0) {
-        ctx->err = "nrrt_render: bad camera or output pointer";
-        return NRRT_ERR_INVALID;
-    }
-    nrrt_render_opts o;
-    std::memset(&o, 0, sizeof o);
-    if (opts_in) o = *opts_in;
-    if (o.world == 0) o.world = 1;
-    if (o.rank >= o.world) {
-        ctx->err = "nrrt_render: rank >= world";
-        return NRRT_ERR_INVALID;
-    }
-    if (o.rows_per_block == 0) o.rows_per_block = 8;
-    CK(cudaSetDevice(ctx->device));
+uint32_t nrrt_work_items(uint32_t width, uint32_t height, uint32_t samples_per_pixel, uint32_t rank, uint32_t world,
+                         uint32_t rows_per_block, uint32_t first, uint32_t n, uint32_t* out) {
+    return nrrt_pass_items(width, height, samples_per_pixel, rank, world, rows_per_block, 0, 0xFFFFFFFFu, first, n, out);
+}
 
-    const uint32_t W = cam->width, H = cam->height;
-    const uint64_t total_pixels = (uint64_t)W * H;
-    if (total_pixels > 0x7FFFFFFFull) {
-        ctx->err = "image too large";
-        return NRRT_ERR_LIMIT;
-    }
-    nrrt_camera c = *cam;
-    if (c.samples_per_pixel < 1) c.samples_per_pixel = 1;  // camera.rs:104
-
+// Renders chunks [c0, c1) of every pixel rank o.rank owns (o.world >= 1, o.rows_per_block >= 1) into the scratch
+// partials and resolves them (k_resolve) onto acc (may be null) and, divided by `samples`, into the image *fb (may be
+// null; with fb_scratch a full-size image is carved in the scratch and returned in *fb): the body of nrrt_render (all
+// chunks) and of nrrt_accum_render (a pass).  Picks the design, carves the scratch, launches, and fills stats.
+static int render_chunks(nrrt_ctx* ctx, const nrrt_camera& c, nrrt_render_opts o, uint32_t c0, uint32_t c1, double* acc,
+                         double samples, float** fb, bool fb_scratch, bool packed, nrrt_progress_fn progress, void* user,
+                         nrrt_render_stats* stats, const char* who) {
+    const uint32_t W = c.width, H = c.height;
     RenderParams P;
     P.key = make_uint2((uint32_t)o.seed, (uint32_t)(o.seed >> 32));
-    if (const char* why = work_item_params(P, W, H, c.samples_per_pixel, o.rank, o.world, o.rows_per_block)) {
-        ctx->err = why;
+    if (const char* why = work_item_params(P, W, H, c.samples_per_pixel, o.rank, o.world, o.rows_per_block, c0, c1)) {
+        ctx->err = std::string(who) + ": " + why;
         return std::strstr(why, "internal") ? NRRT_ERR_INVALID : NRRT_ERR_LIMIT;
     }
     const uint64_t n_items64 = P.n_items;
     const uint32_t want_slots = o.max_slots ? o.max_slots : (1u << 21);
     P.n_slots = (uint32_t)std::min<uint64_t>(n_items64, want_slots);
 
-    const bool out_dev = (o.flags & NRRT_RENDER_OUT_DEVICE) != 0;
-    const bool packed = (o.flags & NRRT_RENDER_OUT_PACKED) != 0;
     const bool counting = (o.flags & NRRT_RENDER_COUNT) != 0;
     // NRRT_MODE_AUTO: the pooled kernel wins where rays walk many nodes (measured on B200: 6319-node teapot 2045 vs
     // 1391 Mrays/s, Cornell box + teapot 1894 vs 1480) and loses where shading dominates (487-node sphere field 4209 vs
@@ -1741,7 +1738,7 @@ int nrrt_render(nrrt_ctx* ctx, const nrrt_camera* cam, const nrrt_render_opts* o
         if (const char* e = std::getenv("NRRT_AUTO_MODE")) o.mode = (uint32_t)std::atoi(e);  // developer override
     }
     if (o.mode > NRRT_MODE_POOL) {
-        ctx->err = "nrrt_render: unknown mode";
+        ctx->err = std::string(who) + ": unknown mode";
         return NRRT_ERR_INVALID;
     }
     // (instance chains are packed as 16-bit indices in the pooled kernel's slot state: larger scenes use the fused kernel)
@@ -1767,7 +1764,7 @@ int nrrt_render(nrrt_ctx* ctx, const nrrt_camera* cam, const nrrt_render_opts* o
         P.n_slots = (uint32_t)std::min<uint64_t>(n_items64, o.max_slots ? std::min<uint64_t>(o.max_slots, resident) : resident);
     }
     P.n_warps = pooled ? (P.n_slots + NRRT_POOL_NS - 1) / NRRT_POOL_NS : (P.n_slots + 31) / 32;
-    const size_t fb_bytes = (size_t)total_pixels * 3 * sizeof(float);
+    const size_t fb_bytes = (size_t)W * H * 3 * sizeof(float);
     const size_t n = P.n_slots;
     // scratch layout
     size_t off = 0;
@@ -1776,7 +1773,7 @@ int nrrt_render(nrrt_ctx* ctx, const nrrt_camera* cam, const nrrt_render_opts* o
         off += (bytes + 255) & ~(size_t)255;
         return at;
     };
-    size_t o_fb = out_dev ? 0 : carve(fb_bytes);
+    size_t o_fb = fb_scratch ? carve(fb_bytes) : 0;
     size_t o_part = carve((size_t)P.n_items * 3 * sizeof(double));
     size_t o_cold = 0;
     if (pooled) {
@@ -1803,8 +1800,8 @@ int nrrt_render(nrrt_ctx* ctx, const nrrt_camera* cam, const nrrt_render_opts* o
     if (off > ctx->scratch_bytes) {  // say what is needed instead of failing inside cudaMalloc
         size_t free_b = 0, total_b = 0;
         if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess && off > free_b + ctx->scratch_bytes) {
-            ctx->err = "nrrt_render: needs " + std::to_string(off >> 20) + " MiB of device scratch (" +
-                       std::to_string(P.n_items) + " work items x 24 B + framebuffer), " +
+            ctx->err = std::string(who) + ": needs " + std::to_string(off >> 20) + " MiB of device scratch (" +
+                       std::to_string(P.n_items) + " work items x 24 B" + (fb_scratch ? " + framebuffer" : "") + "), " +
                        std::to_string((free_b + ctx->scratch_bytes) >> 20) + " MiB available";
             return NRRT_ERR_LIMIT;
         }
@@ -1812,7 +1809,8 @@ int nrrt_render(nrrt_ctx* ctx, const nrrt_camera* cam, const nrrt_render_opts* o
     int rc = ensure_scratch(ctx, std::max<size_t>(off, 256));
     if (rc != NRRT_OK) return rc;
     char* base = (char*)ctx->scratch;
-    float* d_fb = out_dev ? out_rgb : (float*)(base + o_fb);
+    if (fb_scratch) *fb = (float*)(base + o_fb);
+    float* d_fb = fb ? *fb : nullptr;
     double* d_part = (double*)(base + o_part);
 
     // counters: [0] segments [1] paths [2..4] instrumentation [5] next work item (first n_slots pre-assigned)
@@ -1934,7 +1932,7 @@ int nrrt_render(nrrt_ctx* ctx, const nrrt_camera* cam, const nrrt_render_opts* o
         if (!timing.empty()) extend_ms = sampled / (double)timing.size() * (double)extend_launches;
     }
     if (P.n_owned_pixels) {
-        k_resolve<<<(P.n_owned_pixels + 255) / 256, 256, 0, ctx->stream>>>(c, P, d_part, d_fb, packed);
+        k_resolve<<<(P.n_owned_pixels + 255) / 256, 256, 0, ctx->stream>>>(c, P, d_part, acc, samples, d_fb, packed);
         CK(cudaGetLastError());
         ++launches;
     }
@@ -1958,36 +1956,9 @@ int nrrt_render(nrrt_ctx* ctx, const nrrt_camera* cam, const nrrt_render_opts* o
             std::this_thread::sleep_for(std::chrono::milliseconds(20));
         }
     }
-    if (!out_dev && packed) {
-        if (P.n_owned_pixels)
-            CK(cudaMemcpyAsync(out_rgb, d_fb, (size_t)P.n_owned_pixels * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-    } else if (!out_dev) {
-        // copy only the owned rows back into the caller's full-size buffer
-        const uint32_t R = o.rows_per_block;
-        const size_t row_bytes = (size_t)W * 3 * sizeof(float);
-        if (o.world == 1) {  // one contiguous copy
-            CK(cudaMemcpyAsync(out_rgb, d_fb, fb_bytes, cudaMemcpyDeviceToHost, ctx->stream));
-        } else {
-            // the owned row-blocks sit at a fixed pitch: one strided copy for the full blocks, one for a cut-off last one
-            size_t full_blocks = 0, tail_y0 = 0, tail_rows = 0;
-            for (uint32_t b = o.rank; (uint64_t)b * R < H; b += o.world) {
-                const size_t y0 = (size_t)b * R, rows = std::min<size_t>(R, H - y0);
-                if (rows == R) ++full_blocks;
-                else tail_y0 = y0, tail_rows = rows;
-            }
-            const size_t off0 = (size_t)o.rank * R * row_bytes, pitch = (size_t)o.world * R * row_bytes;
-            if (full_blocks)
-                CK(cudaMemcpy2DAsync((char*)out_rgb + off0, pitch, (char*)d_fb + off0, pitch, R * row_bytes, full_blocks,
-                                     cudaMemcpyDeviceToHost, ctx->stream));
-            if (tail_rows)
-                CK(cudaMemcpyAsync((char*)out_rgb + tail_y0 * row_bytes, (char*)d_fb + tail_y0 * row_bytes, tail_rows * row_bytes,
-                                   cudaMemcpyDeviceToHost, ctx->stream));
-        }
-    }
     unsigned long long hc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     CK(cudaMemcpyAsync(hc, ctx->d_counters, sizeof hc, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
-    if (progress) progress(P.n_owned_pixels, P.n_owned_pixels, user);
     if (stats) {
         float ms = 0.f;
         CK(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
@@ -2006,6 +1977,257 @@ int nrrt_render(nrrt_ctx* ctx, const nrrt_camera* cam, const nrrt_render_opts* o
         stats->inst_misses = hc[7];
     }
     return NRRT_OK;
+}
+
+// The rows rank o.rank owns, from the device image d_fb (full-size, or packed) to the caller's host buffer.
+static int copy_owned_rows(nrrt_ctx* ctx, const nrrt_render_opts& o, uint32_t W, uint32_t H, bool packed,
+                           const float* d_fb, float* out_rgb) {
+    const uint32_t R = o.rows_per_block;
+    const size_t row_bytes = (size_t)W * 3 * sizeof(float);
+    if (packed) {
+        const size_t rows = owned_rows(H, o.rank, o.world, R);
+        if (rows) CK(cudaMemcpyAsync(out_rgb, d_fb, rows * row_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    } else if (o.world == 1) {  // one contiguous copy
+        CK(cudaMemcpyAsync(out_rgb, d_fb, (size_t)H * row_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    } else {
+        // the owned row-blocks sit at a fixed pitch: one strided copy for the full blocks, one for a cut-off last one
+        size_t full_blocks = 0, tail_y0 = 0, tail_rows = 0;
+        for (uint32_t b = o.rank; (uint64_t)b * R < H; b += o.world) {
+            const size_t y0 = (size_t)b * R, rows = std::min<size_t>(R, H - y0);
+            if (rows == R) ++full_blocks;
+            else tail_y0 = y0, tail_rows = rows;
+        }
+        const size_t off0 = (size_t)o.rank * R * row_bytes, pitch = (size_t)o.world * R * row_bytes;
+        if (full_blocks)
+            CK(cudaMemcpy2DAsync((char*)out_rgb + off0, pitch, (const char*)d_fb + off0, pitch, R * row_bytes, full_blocks,
+                                 cudaMemcpyDeviceToHost, ctx->stream));
+        if (tail_rows)
+            CK(cudaMemcpyAsync((char*)out_rgb + tail_y0 * row_bytes, (const char*)d_fb + tail_y0 * row_bytes,
+                               tail_rows * row_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    }
+    CK(cudaStreamSynchronize(ctx->stream));
+    return NRRT_OK;
+}
+
+// nrrt_render_opts with the defaults filled in, or the reason they cannot be used
+static const char* default_opts(const nrrt_render_opts* in, nrrt_render_opts& o) {
+    std::memset(&o, 0, sizeof o);
+    if (in) o = *in;
+    if (o.world == 0) o.world = 1;
+    if (o.rank >= o.world) return "rank >= world";
+    if (o.rows_per_block == 0) o.rows_per_block = 8;
+    return nullptr;
+}
+
+int nrrt_render(nrrt_ctx* ctx, const nrrt_camera* cam, const nrrt_render_opts* opts_in, float* out_rgb,
+                nrrt_progress_fn progress, void* user, nrrt_render_stats* stats) {
+    if (!ctx) return NRRT_ERR_INVALID;
+    if (!ctx->has_scene) {
+        ctx->err = "nrrt_render before nrrt_scene_upload";
+        return NRRT_ERR_NO_SCENE;
+    }
+    if (!cam || !out_rgb || cam->width == 0 || cam->height == 0) {
+        ctx->err = "nrrt_render: bad camera or output pointer";
+        return NRRT_ERR_INVALID;
+    }
+    nrrt_render_opts o;
+    if (const char* why = default_opts(opts_in, o)) {
+        ctx->err = std::string("nrrt_render: ") + why;
+        return NRRT_ERR_INVALID;
+    }
+    CK(cudaSetDevice(ctx->device));
+    if ((uint64_t)cam->width * cam->height > 0x7FFFFFFFull) {
+        ctx->err = "image too large";
+        return NRRT_ERR_LIMIT;
+    }
+    nrrt_camera c = *cam;
+    if (c.samples_per_pixel < 1) c.samples_per_pixel = 1;  // camera.rs:104
+    const bool out_dev = (o.flags & NRRT_RENDER_OUT_DEVICE) != 0;
+    const bool packed = (o.flags & NRRT_RENDER_OUT_PACKED) != 0;
+    float* d_fb = out_dev ? out_rgb : nullptr;
+    nrrt_render_stats st;
+    int rc = render_chunks(ctx, c, o, 0, 0xFFFFFFFFu, nullptr, (double)c.samples_per_pixel, &d_fb, !out_dev, packed,
+                           progress, user, &st, "nrrt_render");
+    if (rc != NRRT_OK) return rc;
+    if (!out_dev && (rc = copy_owned_rows(ctx, o, c.width, c.height, packed, d_fb, out_rgb)) != NRRT_OK) return rc;
+    if (progress) progress(st.pixels, st.pixels, user);
+    if (stats) *stats = st;
+    return NRRT_OK;
+}
+
+// ---- progressive rendering: one frame rendered in passes of whole chunks, summed into a persistent f64 accumulator
+struct nrrt_accum {
+    nrrt_ctx* ctx = nullptr;
+    nrrt_camera cam;                // samples_per_pixel >= 1
+    nrrt_render_opts opts;          // defaults filled in; flags: NRRT_RENDER_COUNT at most
+    uint64_t scene_gen = 0;         // the context's scene this frame belongs to
+    std::vector<uint32_t> starts;   // nrrt_chunk_starts: n_chunks + 1 values
+    uint32_t chunks_done = 0;
+    size_t n_sums = 0;              // 3 x owned pixels
+    double* d_sum = nullptr;        // running per-pixel sums, owned rows packed: [j][x][3]
+};
+
+// the accumulator's context is usable and still holds the scene the accumulator was created for
+static int accum_check(const nrrt_accum* a, const char* who) {
+    if (!a || !a->ctx) return NRRT_ERR_INVALID;
+    nrrt_ctx* ctx = a->ctx;
+    if (!ctx->has_scene || ctx->scene_gen != a->scene_gen) {
+        ctx->err = std::string(who) + ": the context's scene was replaced after nrrt_accum_create";
+        return NRRT_ERR_NO_SCENE;
+    }
+    CK(cudaSetDevice(ctx->device));
+    return NRRT_OK;
+}
+
+int nrrt_accum_create(nrrt_ctx* ctx, const nrrt_camera* cam, const nrrt_render_opts* opts_in, nrrt_accum** out) {
+    if (!ctx || !out) return NRRT_ERR_INVALID;
+    *out = nullptr;
+    if (!ctx->has_scene) {
+        ctx->err = "nrrt_accum_create before nrrt_scene_upload";
+        return NRRT_ERR_NO_SCENE;
+    }
+    if (!cam || cam->width == 0 || cam->height == 0) {
+        ctx->err = "nrrt_accum_create: bad camera";
+        return NRRT_ERR_INVALID;
+    }
+    nrrt_render_opts o;
+    if (const char* why = default_opts(opts_in, o)) {
+        ctx->err = std::string("nrrt_accum_create: ") + why;
+        return NRRT_ERR_INVALID;
+    }
+    if (o.mode > NRRT_MODE_AUTO) {
+        ctx->err = "nrrt_accum_create: unknown mode";
+        return NRRT_ERR_INVALID;
+    }
+    o.flags &= NRRT_RENDER_COUNT;  // the output flags belong to nrrt_accum_image
+    if ((uint64_t)cam->width * cam->height > 0x7FFFFFFFull) {
+        ctx->err = "image too large";
+        return NRRT_ERR_LIMIT;
+    }
+    CK(cudaSetDevice(ctx->device));
+    nrrt_accum* a = new nrrt_accum;
+    a->ctx = ctx;
+    a->cam = *cam;
+    if (a->cam.samples_per_pixel < 1) a->cam.samples_per_pixel = 1;  // camera.rs:104
+    a->opts = o;
+    a->scene_gen = ctx->scene_gen;
+    a->starts.resize(64);
+    const uint32_t n_chunks = nrrt_chunk_starts(a->cam.samples_per_pixel, (uint64_t)cam->width * cam->height,
+                                                a->starts.data(), (uint32_t)a->starts.size());
+    a->starts.resize(n_chunks + 1);
+    a->n_sums = (size_t)owned_rows(cam->height, o.rank, o.world, o.rows_per_block) * cam->width * 3;
+    const size_t bytes = std::max<size_t>(a->n_sums, 1) * sizeof(double);
+    cudaError_t e = cudaMalloc((void**)&a->d_sum, bytes);
+    if (e == cudaSuccess) e = cudaMemsetAsync(a->d_sum, 0, bytes, ctx->stream);
+    if (e != cudaSuccess) {
+        ctx->err = std::string("nrrt_accum_create: ") + cudaGetErrorString(e);
+        if (a->d_sum) cudaFree(a->d_sum);
+        delete a;
+        return NRRT_ERR_CUDA;
+    }
+    *out = a;
+    return NRRT_OK;
+}
+
+int nrrt_accum_render(nrrt_accum* a, uint32_t min_samples, nrrt_render_stats* stats) {
+    int rc = accum_check(a, "nrrt_accum_render");
+    if (rc != NRRT_OK) return rc;
+    const uint32_t n_chunks = (uint32_t)a->starts.size() - 1;
+    uint32_t c1 = a->chunks_done;
+    while (c1 < n_chunks && a->starts[c1] < min_samples) ++c1;  // whole chunks, up to spp
+    nrrt_render_stats st;
+    std::memset(&st, 0, sizeof st);
+    st.pixels = (uint32_t)(a->n_sums / 3);
+    if (c1 > a->chunks_done) {
+        rc = render_chunks(a->ctx, a->cam, a->opts, a->chunks_done, c1, a->d_sum, 0.0, nullptr, false, false, nullptr,
+                           nullptr, &st, "nrrt_accum_render");
+        if (rc != NRRT_OK) return rc;
+        a->chunks_done = c1;
+    }
+    if (stats) *stats = st;
+    return NRRT_OK;
+}
+
+uint32_t nrrt_accum_samples(const nrrt_accum* a) { return a ? a->starts[a->chunks_done] : 0; }
+
+int nrrt_accum_image(nrrt_accum* a, float* out_rgb, uint32_t flags) {
+    int rc = accum_check(a, "nrrt_accum_image");
+    if (rc != NRRT_OK) return rc;
+    nrrt_ctx* ctx = a->ctx;
+    if (!out_rgb || a->chunks_done == 0) {
+        ctx->err = out_rgb ? "nrrt_accum_image: no samples rendered yet" : "nrrt_accum_image: NULL output";
+        return NRRT_ERR_INVALID;
+    }
+    const nrrt_camera& c = a->cam;
+    const nrrt_render_opts& o = a->opts;
+    RenderParams P;  // owned_pixel's fields; no chunks: k_resolve divides the sums as they are
+    P.key = make_uint2(0, 0);
+    if (const char* why = work_item_params(P, c.width, c.height, c.samples_per_pixel, o.rank, o.world, o.rows_per_block,
+                                           a->chunks_done, a->chunks_done)) {
+        ctx->err = std::string("nrrt_accum_image: ") + why;
+        return NRRT_ERR_INVALID;
+    }
+    const bool out_dev = (flags & NRRT_RENDER_OUT_DEVICE) != 0, packed = (flags & NRRT_RENDER_OUT_PACKED) != 0;
+    float* d_fb = out_rgb;
+    if (!out_dev) {
+        if ((rc = ensure_scratch(ctx, std::max<size_t>((size_t)c.width * c.height * 3 * sizeof(float), 256))) != NRRT_OK)
+            return rc;
+        d_fb = (float*)ctx->scratch;
+    }
+    if (P.n_owned_pixels) {
+        k_resolve<<<(P.n_owned_pixels + 255) / 256, 256, 0, ctx->stream>>>(c, P, nullptr, a->d_sum,
+                                                                           (double)a->starts[a->chunks_done], d_fb, packed);
+        CK(cudaGetLastError());
+    }
+    if (out_dev) {
+        CK(cudaStreamSynchronize(ctx->stream));
+        return NRRT_OK;
+    }
+    return copy_owned_rows(ctx, o, c.width, c.height, packed, d_fb, out_rgb);
+}
+
+int nrrt_accum_save(const nrrt_accum* a, double* sums, uint32_t* samples_done) {
+    int rc = accum_check(a, "nrrt_accum_save");
+    if (rc != NRRT_OK) return rc;
+    nrrt_ctx* ctx = a->ctx;
+    if ((!sums && a->n_sums) || !samples_done) {
+        ctx->err = "nrrt_accum_save: NULL output";
+        return NRRT_ERR_INVALID;
+    }
+    if (a->n_sums) CK(cudaMemcpyAsync(sums, a->d_sum, a->n_sums * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    *samples_done = a->starts[a->chunks_done];
+    return NRRT_OK;
+}
+
+int nrrt_accum_restore(nrrt_accum* a, const double* sums, uint32_t samples_done) {
+    int rc = accum_check(a, "nrrt_accum_restore");
+    if (rc != NRRT_OK) return rc;
+    nrrt_ctx* ctx = a->ctx;
+    const auto at = std::find(a->starts.begin(), a->starts.end(), samples_done);
+    if (at == a->starts.end()) {
+        ctx->err = "nrrt_accum_restore: " + std::to_string(samples_done) + " samples is not a chunk boundary of this frame"
+                   " (nrrt_chunk_starts)";
+        return NRRT_ERR_INVALID;
+    }
+    if (!sums && a->n_sums) {
+        ctx->err = "nrrt_accum_restore: NULL sums";
+        return NRRT_ERR_INVALID;
+    }
+    if (a->n_sums) CK(cudaMemcpyAsync(a->d_sum, sums, a->n_sums * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    a->chunks_done = (uint32_t)(at - a->starts.begin());
+    return NRRT_OK;
+}
+
+void nrrt_accum_free(nrrt_accum* a) {
+    if (!a) return;
+    if (a->ctx && a->d_sum) {
+        cudaSetDevice(a->ctx->device);
+        cudaStreamSynchronize(a->ctx->stream);
+        cudaFree(a->d_sum);
+    }
+    delete a;
 }
 
 // rows of one rank, packed -> their places in the full image (device-output form of nrrt_render_multi)

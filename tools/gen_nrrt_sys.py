@@ -47,6 +47,7 @@ FUNCTIONS = '''
 pub enum nrrt_ctx {}
 pub enum nrrt_host_scene {}
 pub enum nrrt_loaded_scene {}
+pub enum nrrt_accum {}
 pub type nrrt_progress_fn = Option<unsafe extern "C" fn(pixels_done: u64, pixels_total: u64, user: *mut c_void)>;
 
 pub const NRRT_OK: c_int = 0;
@@ -125,6 +126,17 @@ extern "C" {
     pub fn nrrt_chunk_starts(samples_per_pixel: u32, total_pixels: u64, starts: *mut u32, max: u32) -> u32;
     pub fn nrrt_work_items(width: u32, height: u32, samples_per_pixel: u32, rank: u32, world: u32, rows_per_block: u32,
                            first: u32, n: u32, out: *mut u32) -> u32;
+    pub fn nrrt_pass_items(width: u32, height: u32, samples_per_pixel: u32, rank: u32, world: u32, rows_per_block: u32,
+                           c0: u32, c1: u32, first: u32, n: u32, out: *mut u32) -> u32;
+    // progressive rendering: one frame in passes of whole chunks, summed into per-pixel f64 sums on the device
+    pub fn nrrt_accum_create(ctx: *mut nrrt_ctx, camera: *const nrrt_camera, opts: *const nrrt_render_opts,
+                             out: *mut *mut nrrt_accum) -> c_int;
+    pub fn nrrt_accum_render(accum: *mut nrrt_accum, min_samples: u32, stats: *mut nrrt_render_stats) -> c_int;
+    pub fn nrrt_accum_samples(accum: *const nrrt_accum) -> u32;
+    pub fn nrrt_accum_image(accum: *mut nrrt_accum, out_rgb: *mut f32, flags: u32) -> c_int;
+    pub fn nrrt_accum_save(accum: *const nrrt_accum, sums: *mut f64, samples_done: *mut u32) -> c_int;
+    pub fn nrrt_accum_restore(accum: *mut nrrt_accum, sums: *const f64, samples_done: u32) -> c_int;
+    pub fn nrrt_accum_free(accum: *mut nrrt_accum);
     pub fn nrrt_abi_sizeof(which: c_int) -> usize;
 }
 '''
