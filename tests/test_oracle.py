@@ -180,6 +180,41 @@ def test_translate_rotate_scale_semantics():
     assert np.allclose(h["normal"], [0.5, math.sqrt(0.75), 0.0], atol=1e-12)
 
 
+def test_wrapper_chain_four_levels_deep():
+    """Translate / Scale / Translate / Scale nested four instance levels deep (each level's group also holds a far-away
+    filler, so no group forwards to its only child), around a unit sphere and a tilted quad.  Every value below is
+    exact in f64: the ray goes in through o - offset (translate.rs:37-49) and the inverse scale matrix
+    (scale.rs:49, 68-80: halving, quartering, doubling), the point comes back through the scale matrix and + offset.
+    The normal is the OBJECT-space normal at both Scale levels (quirk Q4, scale.rs:68-80 leaves it alone): an inverse
+    transpose through the non-uniform scales would tilt the quad's (0, -1, 1)/sqrt(2) to (0, -4, 1)/sqrt(17)."""
+    g = SceneGraph()
+    t = g.add_texture(kind=A.TEX_SOLID, color=(1, 1, 1))
+    m = g.add_material(A.MAT_LAMBERTIAN, t)
+    sphere = g.add_object(A.OBJ_SPHERE, m, v=(0, 0, 0, 1))
+    quad = g.add_object(A.OBJ_QUAD, m, v=(3, 0, 0, 1, 0, 0, 0, 1, 1))       # normal (0, -1, 1)/sqrt(2)
+    inner = g.add_object(A.OBJ_GROUP, children=[sphere, quad])
+    for kind, v in ((A.OBJ_SCALE, (1, 0.5, 1)), (A.OBJ_TRANSLATE, (0, 1, 0)), (A.OBJ_SCALE, (2, 2, 4)),
+                    (A.OBJ_TRANSLATE, (4, 0, 0))):                          # innermost (level 3) first
+        filler = g.add_object(A.OBJ_SPHERE, m, v=(-100, 0, 0, 1))
+        inner = g.add_object(A.OBJ_GROUP, children=[g.add_object(kind, children=[inner], v=v), filler])
+    g.root = inner
+    # world -> object: (4, 2, 20) - (4, 0, 0) = (0, 2, 20); / (2, 2, 4) = (0, 1, 5); - (0, 1, 0) = (0, 0, 5);
+    # / (1, .5, 1) = (0, 0, 5).  Direction (0, 0, -1) -> (0, 0, -.25).  Sphere (sphere.rs:114-135): a = 1/16,
+    # h = 1.25, c = 24, disc = 1/16, t = (1.25 - .25) * 16 = 16.  Object point (0, 0, 1) -> (0, 0, 1) -> (0, 1, 1)
+    # -> (0, 2, 4) -> (4, 2, 4) = (4, 2, 20) + 16 (0, 0, -1).
+    h = one(g, (4, 2, 20), (0, 0, -1))
+    assert h["object"] == sphere and h["t"] == 16.0 and h["front_face"] == 1
+    assert h["point"].tolist() == [4.0, 2.0, 4.0] and h["normal"].tolist() == [0.0, 0.0, 1.0]
+    # object ray (3.5, .5, 5) + t (0, 0, -.25) meets the quad's plane z = y at z = .5, t = 18, alpha = beta = .5;
+    # back out: (3.5, .25, .5) -> (3.5, 1.25, .5) -> (7, 2.5, 2) -> (11, 2.5, 2) = (11, 2.5, 20) + 18 (0, 0, -1)
+    h = one(g, (11, 2.5, 20), (0, 0, -1))
+    s = 1.0 / math.sqrt(2.0)
+    assert h["object"] == quad and abs(h["t"] - 18.0) < 1e-12 and h["front_face"] == 1
+    assert np.allclose(h["point"], [11.0, 2.5, 2.0], rtol=0, atol=1e-12)
+    assert np.allclose(h["normal"], [0.0, -s, s], rtol=0, atol=1e-15)
+    assert np.allclose(h["uv"], [0.5, 0.5], rtol=0, atol=1e-12)
+
+
 # ---------------------------------------------------------------- camera + shading quirks through tiny renders
 def _render_const(graph, **cam):
     for k, v in cam.items():
