@@ -522,9 +522,62 @@ int nrrt_accum_save(const nrrt_accum* accum, double* sums, uint32_t* samples_don
 int nrrt_accum_restore(nrrt_accum* accum, const double* sums, uint32_t samples_done);
 void nrrt_accum_free(nrrt_accum* accum);
 
-/* sizeof() of the ABI structs as compiled (which = 0..18: object, material, texture,
+/* ---- adaptive sampling -------------------------------------------------------------------------------------------
+ * An adaptive frame is a progressive frame created with tolerances.  Its passes render the next whole chunks, as
+ * above, but only for the pixels still ACTIVE.  After a pass every pixel that took part is tested; a pixel that passes
+ * the test is RETIRED: its sum, second moment and sample count never change again.  Per owned pixel the handle keeps
+ *   S  the f64 RGB sum of its samples (as above),
+ *   Q  the f64 RGB sum over its chunks of P_c * P_c / n_c (P_c: chunk c's partial sum, n_c: its sample count), added in
+ *      chunk order by the thread that adds P_c to S, without FMA contraction: Q = Q + (p * p) / n_c, each step rounded,
+ *   N  its sample count (a nrrt_chunk_starts boundary) and K its chunk count.
+ * The test (nrrt_adaptive_converged), evaluated in f64 per channel in this order:
+ *   m = S / N;  d = max(Q - (S * S) / N, 0);  e2 = d / ((K - 1) * N);  tol = abs_error + rel_error * |m|
+ * e2 is the squared standard error of the mean estimated from the chunks as batch means (E[sum n_c (m_c - m)^2] =
+ * (K - 1) sigma^2 holds for unequal batches too).  A pixel is converged iff K >= 2, N >= min_samples, a tolerance is
+ * positive, and e2 <= tol * tol in all three channels (NaN compares false).  Tolerance 0 therefore never retires a
+ * pixel: such a frame is nrrt_render's image bit for bit.
+ * A pixel's value is S / N as f32: the CPU oracle's render_chunked over the chunks it received, bit for bit.  Decisions
+ * are made at pass ends only, so the result depends on the scene, camera, seed, tolerances and pass schedule, and not on
+ * the kernel design, slot count or partition.  On an adaptive handle:
+ *   - nrrt_accum_render renders the active pixels' next chunks up to min_samples, then tests them; its stats count
+ *     what ran (stats.pixels = the active pixels of the pass);
+ *   - nrrt_accum_samples is the frame's chunk boundary: retired pixels sit below it;
+ *   - nrrt_accum_image divides each pixel by its own N;
+ *   - nrrt_accum_save / _restore fail with NRRT_ERR_INVALID (use the _adaptive_ pair). */
+typedef struct nrrt_adaptive_opts {
+    double rel_error, abs_error; /* >= 0 and finite, else NRRT_ERR_INVALID */
+    uint32_t min_samples;        /* a pixel is tested only from this many samples (and two chunks) on */
+    uint32_t _pad;
+} nrrt_adaptive_opts;
+int nrrt_accum_create_adaptive(nrrt_ctx* ctx, const nrrt_camera* camera, const nrrt_render_opts* opts,
+                               const nrrt_adaptive_opts* adaptive, nrrt_accum** out);
+/* Pixels of this rank still active (0 = frame finished; every owned pixel before the first pass).  0 for a handle
+ * that is not adaptive. */
+uint32_t nrrt_accum_active(const nrrt_accum* accum);
+/* N per pixel (u32), laid out as nrrt_accum_image lays out one channel (flags NRRT_RENDER_OUT_DEVICE / _PACKED). */
+int nrrt_accum_sample_map(nrrt_accum* accum, uint32_t* out, uint32_t flags);
+/* sqrt(e2) per channel as f32 (+inf where K < 2), laid out as nrrt_accum_image. */
+int nrrt_accum_error_image(nrrt_accum* accum, float* out_rgb, uint32_t flags);
+/* Host copy of S, Q (stats.pixels x 3 f64 each) and N (stats.pixels u32), owned rows packed. */
+int nrrt_accum_adaptive_save(const nrrt_accum* accum, double* sums, double* sumsq, uint32_t* samples);
+/* Loads what nrrt_accum_adaptive_save wrote into an adaptive handle of the same frame.  Every N must be a chunk
+ * boundary of the frame, at least one chunk, and one value below the largest N only for a pixel that passes the test
+ * (a retired pixel); the active set is rebuilt by re-evaluating the test.  NRRT_ERR_INVALID otherwise. */
+int nrrt_accum_adaptive_restore(nrrt_accum* accum, const double* sums, const double* sumsq, const uint32_t* samples);
+/* The test above on one pixel's state (1 = converged).  For tests and bindings. */
+int nrrt_adaptive_converged(const double S[3], const double Q[3], uint32_t samples, uint32_t chunks,
+                            const nrrt_adaptive_opts* adaptive);
+/* nrrt_pass_items for a pass over the owned pixels active[0 .. n_active) only (owned-pixel indices in the order
+ * nrrt_pass_items visits a chunk's pixels, strictly ascending, each below the owned pixel count): inside each chunk the
+ * items follow the list.  Returns the number of items, 0 also for a list that breaks those rules. */
+uint32_t nrrt_pass_items_active(uint32_t width, uint32_t height, uint32_t samples_per_pixel, uint32_t rank,
+                                uint32_t world, uint32_t rows_per_block, uint32_t c0, uint32_t c1,
+                                const uint32_t* active, uint32_t n_active, uint32_t first, uint32_t n, uint32_t* out);
+
+/* sizeof() of the ABI structs as compiled (which = 0..19: object, material, texture,
  * image, graph_desc, camera_config, camera, node, box, xform, instance, scene_desc, hit, trace_stats,
- * render_opts, render_stats, camera_file, wnode, hit_compact) so a binding can verify its mirror of this header. */
+ * render_opts, render_stats, camera_file, wnode, hit_compact, adaptive_opts) so a binding can verify its mirror of this
+ * header. */
 size_t nrrt_abi_sizeof(int which);
 
 #ifdef __cplusplus

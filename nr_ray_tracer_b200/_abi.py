@@ -141,6 +141,10 @@ class RenderStats(C.Structure):
                 ("inst_misses", u64)]
 
 
+class AdaptiveOpts(C.Structure):
+    _fields_ = [("rel_error", f64), ("abs_error", f64), ("min_samples", u32), ("_pad", u32)]
+
+
 class CameraFile(C.Structure):
     _fields_ = [("present", u32), ("width", u32), ("height", u32), ("samples_per_pixel", u32), ("ray_max_bounces", u32),
                 ("_pad", u32), ("aspect_ratio", f64), ("background", f64 * 3), ("look_at", f64 * 3),

@@ -86,6 +86,19 @@ def lib() -> C.CDLL:
         L.nrrt_accum_save.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(C.c_uint32)]
         L.nrrt_accum_restore.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32]
         L.nrrt_accum_free.argtypes = [C.c_void_p]
+        L.nrrt_accum_create_adaptive.argtypes = [C.c_void_p, C.POINTER(A.Camera), C.POINTER(A.RenderOpts),
+                                                 C.POINTER(A.AdaptiveOpts), C.POINTER(C.c_void_p)]
+        L.nrrt_accum_active.restype = C.c_uint32
+        L.nrrt_accum_active.argtypes = [C.c_void_p]
+        L.nrrt_accum_sample_map.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32]
+        L.nrrt_accum_error_image.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32]
+        L.nrrt_accum_adaptive_save.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.nrrt_accum_adaptive_restore.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.nrrt_adaptive_converged.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32,
+                                              C.POINTER(A.AdaptiveOpts)]
+        L.nrrt_pass_items_active.restype = C.c_uint32
+        L.nrrt_pass_items_active.argtypes = [C.c_uint32] * 8 + [C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32,
+                                                                 C.POINTER(C.c_uint32)]
         L.nrrt_abi_sizeof.restype = C.c_size_t
         L.nrrt_abi_sizeof.argtypes = [C.c_int]
         _lib = L
@@ -94,7 +107,7 @@ def lib() -> C.CDLL:
 
 ABI_STRUCTS = [A.Object, A.Material, A.Texture, A.Image, A.GraphDesc, A.CameraConfig, A.Camera, A.Node, A.Box,
                A.Xform, A.Instance, A.SceneDesc, A.Hit, A.TraceStats, A.RenderOpts, A.RenderStats, A.CameraFile, A.WNode,
-               A.HitCompact]
+               A.HitCompact, A.AdaptiveOpts]
 
 
 def chunk_starts(samples_per_pixel: int, total_pixels: int):
@@ -126,6 +139,39 @@ def pass_items(width: int, height: int, samples_per_pixel: int, c0: int, c1: int
     if n:
         lib().nrrt_pass_items(*args, 0, n, out.ctypes.data_as(C.POINTER(C.c_uint32)))
     return out
+
+
+def pass_items_active(width: int, height: int, samples_per_pixel: int, c0: int, c1: int, active, rank: int = 0,
+                      world: int = 1, rows_per_block: int = 8) -> np.ndarray:
+    """pass_items for an adaptive pass over the owned pixels listed in `active` (owned-pixel indices, i.e. positions in
+    a chunk of pass_items, strictly ascending) in hand-out order (nrrt_pass_items_active)."""
+    act = np.ascontiguousarray(active, dtype=np.uint32)
+    args = (width, height, samples_per_pixel, rank, world, rows_per_block, c0, c1, C.c_void_p(act.ctypes.data), len(act))
+    n = lib().nrrt_pass_items_active(*args, 0, 0, None)
+    out = np.zeros((n, 4), dtype=np.uint32)
+    if n:
+        lib().nrrt_pass_items_active(*args, 0, n, out.ctypes.data_as(C.POINTER(C.c_uint32)))
+    return out
+
+
+def adaptive_opts(rel_error: float, abs_error: float = 0.0, min_samples: int = 0) -> A.AdaptiveOpts:
+    return A.AdaptiveOpts(rel_error=float(rel_error), abs_error=float(abs_error), min_samples=int(min_samples))
+
+
+def adaptive_converged(S, Q, samples: int, chunks: int, rel_error: float, abs_error: float = 0.0,
+                       min_samples: int = 0) -> bool:
+    """The adaptive test on one pixel's state (nrrt_adaptive_converged): S and Q are its 3 f64 sums."""
+    S = np.ascontiguousarray(S, dtype=np.float64)
+    Q = np.ascontiguousarray(Q, dtype=np.float64)
+    assert S.size == 3 and Q.size == 3
+    t = adaptive_opts(rel_error, abs_error, min_samples)
+    return bool(lib().nrrt_adaptive_converged(S.ctypes.data, Q.ctypes.data, int(samples), int(chunks), C.byref(t)))
+
+
+def default_min_samples(samples_per_pixel: int, total_pixels: int) -> int:
+    """The first chunk boundary at or above spp / 8: where an adaptive frame starts testing pixels by default."""
+    starts = chunk_starts(samples_per_pixel, total_pixels)
+    return min(s for s in starts if 8 * s >= max(1, samples_per_pixel))
 
 
 def owned_rows(height: int, rank: int = 0, world: int = 1, rows_per_block: int = 0) -> int:
@@ -333,10 +379,11 @@ class Context:
         return (None if out_device_ptr is not None else out), stats
 
     def progressive(self, cam: A.Camera, seed: int = 0, mode: int = A.MODE_AUTO, rank: int = 0, world: int = 1,
-                    rows_per_block: int = 0, max_slots: int = 0) -> "Progressive":
-        """One frame of `cam` rendered in passes (nrrt_accum_*): see Progressive."""
+                    rows_per_block: int = 0, max_slots: int = 0, adaptive: Optional[dict] = None) -> "Progressive":
+        """One frame of `cam` rendered in passes (nrrt_accum_*): see Progressive.  adaptive = {rel_error, abs_error=0.0,
+        min_samples=None} makes it an adaptive frame (min_samples None: the first chunk boundary at or above spp / 8)."""
         return Progressive(self, cam, seed=seed, mode=mode, rank=rank, world=world, rows_per_block=rows_per_block,
-                           max_slots=max_slots)
+                           max_slots=max_slots, adaptive=adaptive)
 
 
     def encode_rgb8(self, image: Optional[np.ndarray] = None, gamma: float = 0.5, device_ptr: Optional[int] = None,
@@ -360,10 +407,15 @@ class Progressive:
     render(min_samples) renders the next chunks until at least that many samples per pixel are done (pass boundaries
     are chunk_starts() boundaries); image() is the frame so far, sums / samples.  The finished frame is
     Context.render's image bit for bit, whatever the passes.  state() / restore() save and resume the sums.
-    Keeps its Context alive; the scene must stay the one uploaded when the frame was created."""
+    Keeps its Context alive; the scene must stay the one uploaded when the frame was created.
+
+    An adaptive frame (adaptive={rel_error, abs_error, min_samples}) renders each pass for the pixels still active only
+    and retires a pixel once its error estimate meets the tolerance (include/nrrt.h): `active` counts the pixels left,
+    sample_map() and error_image() show each pixel's samples and estimated error, image() divides each pixel by its
+    own sample count, and state() / restore() carry (sums, sums of squares, samples)."""
 
     def __init__(self, ctx: Context, cam: A.Camera, seed: int = 0, mode: int = A.MODE_AUTO, rank: int = 0,
-                 world: int = 1, rows_per_block: int = 0, max_slots: int = 0):
+                 world: int = 1, rows_per_block: int = 0, max_slots: int = 0, adaptive: Optional[dict] = None):
         self.ctx = ctx
         self.camera = cam
         self.samples_per_pixel = max(1, cam.samples_per_pixel)
@@ -371,7 +423,19 @@ class Progressive:
         opts = A.RenderOpts(seed=seed, mode=mode, rank=rank, world=world, rows_per_block=rows_per_block,
                             max_slots=max_slots, flags=0)
         h = C.c_void_p()
-        ctx._check(lib().nrrt_accum_create(ctx._h, C.byref(cam), C.byref(opts), C.byref(h)))
+        self.adaptive = None
+        if adaptive is None:
+            ctx._check(lib().nrrt_accum_create(ctx._h, C.byref(cam), C.byref(opts), C.byref(h)))
+        else:
+            unknown = set(adaptive) - {"rel_error", "abs_error", "min_samples"}
+            if unknown or "rel_error" not in adaptive:
+                raise ValueError("adaptive takes rel_error and optionally abs_error and min_samples")
+            ms = adaptive.get("min_samples")
+            if ms is None:
+                ms = default_min_samples(self.samples_per_pixel, cam.width * cam.height)
+            self.adaptive = adaptive_opts(adaptive["rel_error"], adaptive.get("abs_error", 0.0), ms)
+            ctx._check(lib().nrrt_accum_create_adaptive(ctx._h, C.byref(cam), C.byref(opts), C.byref(self.adaptive),
+                                                        C.byref(h)))
         self._h = h
 
     def close(self):
@@ -418,17 +482,63 @@ class Progressive:
         self.ctx._check(lib().nrrt_accum_image(self._h, ptr, flags))
         return None if out_device_ptr is not None else out
 
+    @property
+    def active(self) -> int:
+        """Pixels of an adaptive frame still active (0: the frame is finished); 0 for a plain progressive frame."""
+        return int(lib().nrrt_accum_active(self._h))
+
+    def _map(self, fn, shape, dtype, packed, out_device_ptr):
+        flags = (A.RENDER_OUT_DEVICE if out_device_ptr is not None else 0) | (A.RENDER_OUT_PACKED if packed else 0)
+        if out_device_ptr is not None:
+            self.ctx._check(fn(self._h, C.c_void_p(out_device_ptr), flags))
+            return None
+        out = np.zeros(((self.rows if packed else self.camera.height), self.camera.width) + shape, dtype=dtype)
+        self.ctx._check(fn(self._h, C.c_void_p(out.ctypes.data), flags))
+        return out
+
+    def sample_map(self, packed: bool = False, out_device_ptr: Optional[int] = None) -> Optional[np.ndarray]:
+        """Samples each pixel of an adaptive frame holds, (H, W) uint32 laid out as image()."""
+        return self._map(lib().nrrt_accum_sample_map, (), np.uint32, packed, out_device_ptr)
+
+    def error_image(self, packed: bool = False, out_device_ptr: Optional[int] = None) -> Optional[np.ndarray]:
+        """Estimated standard error of each pixel's mean per channel, (H, W, 3) f32 laid out as image(); +inf where a
+        pixel holds fewer than two chunks."""
+        return self._map(lib().nrrt_accum_error_image, (3,), np.float32, packed, out_device_ptr)
+
     def state(self):
-        """(samples done, f64 sums (owned rows, W, 3) in owned-row order): what restore() takes."""
+        """What restore() takes: (samples done, f64 sums (owned rows, W, 3) in owned-row order), or for an adaptive
+        frame (sums, sums of squares (owned rows, W, 3) f64, samples (owned rows, W) uint32)."""
         sums = np.zeros((self.rows, self.camera.width, 3), dtype=np.float64)
+        if self.adaptive is not None:
+            sumsq = np.zeros_like(sums)
+            samples = np.zeros((self.rows, self.camera.width), dtype=np.uint32)
+            self.ctx._check(lib().nrrt_accum_adaptive_save(self._h, C.c_void_p(sums.ctypes.data),
+                                                           C.c_void_p(sumsq.ctypes.data),
+                                                           C.c_void_p(samples.ctypes.data)))
+            return sums, sumsq, samples
         n = C.c_uint32()
         self.ctx._check(lib().nrrt_accum_save(self._h, C.c_void_p(sums.ctypes.data), C.byref(n)))
         return int(n.value), sums
 
-    def restore(self, samples: int, sums: np.ndarray):
-        """Resumes from state(): `samples` must be a chunk boundary of this frame."""
+    def restore(self, *state):
+        """Resumes from state(): restore(samples, sums), where `samples` must be a chunk boundary of this frame, or for
+        an adaptive frame restore(sums, sumsq, samples)."""
+        npx = self.rows * self.camera.width
+        if self.adaptive is not None:
+            sums, sumsq, samples = state
+            sums = np.ascontiguousarray(sums, dtype=np.float64)
+            sumsq = np.ascontiguousarray(sumsq, dtype=np.float64)
+            samples = np.ascontiguousarray(samples, dtype=np.uint32)
+            if sums.size != npx * 3 or sumsq.size != npx * 3 or samples.size != npx:
+                raise ValueError(f"sums and sumsq must hold {self.rows} x {self.camera.width} x 3 values and samples "
+                                 f"{self.rows} x {self.camera.width}")
+            self.ctx._check(lib().nrrt_accum_adaptive_restore(self._h, C.c_void_p(sums.ctypes.data),
+                                                              C.c_void_p(sumsq.ctypes.data),
+                                                              C.c_void_p(samples.ctypes.data)))
+            return
+        samples, sums = state
         sums = np.ascontiguousarray(sums, dtype=np.float64)
-        if sums.size != self.rows * self.camera.width * 3:
+        if sums.size != npx * 3:
             raise ValueError(f"sums must hold {self.rows} x {self.camera.width} x 3 values")
         self.ctx._check(lib().nrrt_accum_restore(self._h, C.c_void_p(sums.ctypes.data), int(samples)))
 
@@ -489,3 +599,27 @@ class Scene:
                 done = p.samples
                 self.last_stats = p.render(done + 1 if every is None else (done // every + 1) * every)
                 yield p.samples, p.image()
+
+    def render_adaptive(self, rel_error: float, abs_error: float = 0.0, min_samples: Optional[int] = None,
+                        every: Optional[int] = None, **kw):
+        """Scene::render with adaptive sampling: each pixel stops once its estimated standard error is at most
+        abs_error + rel_error * |its mean| (see Progressive).  Yields (samples done, pixels still active, image so far)
+        after each pass; the last image is the finished frame.  every=None: passes end at doubling chunk counts from
+        the first chunk boundary at or above min_samples (each pass ends in a drain of the GPU, so few passes are
+        cheaper); every=N: as in render_progressive.  kw: Context.progressive's options (seed, mode, ...)."""
+        if every is not None and every < 1:
+            raise ValueError("every must be >= 1")
+        ad = {"rel_error": rel_error, "abs_error": abs_error, "min_samples": min_samples}
+        with self.ctx.progressive(self.camera, adaptive=ad, **kw) as p:
+            spp = p.samples_per_pixel
+            starts = chunk_starts(spp, self.camera.width * self.camera.height)
+            k = next((i for i, s in enumerate(starts) if i and s >= p.adaptive.min_samples), len(starts) - 1)
+            while p.active:
+                done = p.samples
+                if every is None:
+                    target = starts[min(k, len(starts) - 1)]
+                    k *= 2
+                else:
+                    target = (done // every + 1) * every
+                self.last_stats = p.render(min(target, spp))
+                yield p.samples, p.active, p.image()

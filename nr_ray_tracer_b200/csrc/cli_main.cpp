@@ -6,11 +6,12 @@
 // Flags and NR_RT_CAMERA_* environment fallbacks follow ray-tracer/src/cli.rs:113-270 (field of view and defocus
 // angle in degrees; image size needs exactly two of width / height / aspect ratio; default output out.png,
 // default gamma 0.5).  Additions: --seed, --mode auto|pool|fused|wavefront|megakernel, --device N, --gpus N,
-// --preview-every N.
+// --preview-every N, --adaptive-error REL [--adaptive-abs-error ABS] [--adaptive-min-samples N].
 // Encoders available without external libraries: .png (stored/uncompressed deflate) and .ppm.
 #include <algorithm>
 #include <cerrno>
 #include <chrono>
+#include <cmath>
 #include <cstdint>
 #include <cstdio>
 #include <cstdlib>
@@ -131,6 +132,16 @@ static void replace_image(const std::string& path, bool png, const uint8_t* rgb,
     }
 }
 
+// A tolerance: a decimal number, whole string, finite and >= 0.
+static bool parse_tolerance(const char* s, double* out) {
+    char* e = nullptr;
+    errno = 0;
+    const double x = std::strtod(s, &e);
+    if (!*s || !e || *e || errno || !std::isfinite(x) || !(x >= 0.0)) return false;
+    *out = x;
+    return true;
+}
+
 // Unsigned decimal integer, whole string, no sign, <= max (clap rejects "-1", "1e3", "" and overflow alike).
 static bool parse_u64(const char* s, uint64_t max, uint64_t* out) {
     if (!s || !*s) return false;
@@ -163,6 +174,13 @@ static void usage() {
         "      --preview-every <N>        render in passes and rewrite the output file whenever another N samples per\n"
         "                                 pixel are done (passes end on whole work chunks; the final image is the same;\n"
         "                                 one GPU only)\n"
+        "      --adaptive-error <REL>     adaptive sampling: stop sampling a pixel once the estimated standard error of\n"
+        "                                 its mean is at most ABS + REL x |mean| in every channel (0: every pixel takes\n"
+        "                                 every sample; the image is then the same as without the flag; one GPU only)\n"
+        "      --adaptive-abs-error <ABS> the absolute part of that tolerance (default 0)\n"
+        "      --adaptive-min-samples <N> test a pixel only from N samples on (default: the first work-chunk boundary at\n"
+        "                                 or above 1/8 of the samples per pixel).  Passes end at doubling chunk counts\n"
+        "                                 from there, or as --preview-every sets them\n"
         "  -v, --verbose                  print timing\n"
         "Every camera option falls back to NR_RT_CAMERA_<NAME> (e.g. NR_RT_CAMERA_SAMPLES_PER_PIXEL).");
 }
@@ -206,7 +224,10 @@ int main(int argc, char** argv) {
     std::string scene_path, output = "out.png", mode = "auto", bvh = "reference";
     bool force = false, verbose = false;
     float gamma = 0.5f;  // constants.rs:1
-    uint64_t seed = 0, preview_every = 0;
+    uint64_t seed = 0, preview_every = 0, adaptive_min = 0;
+    bool adaptive = false, adaptive_min_set = false, adaptive_abs_set = false;
+    nrrt_adaptive_opts ad;
+    std::memset(&ad, 0, sizeof ad);
     int device = 0, gpus = 1;
     if (const char* e = std::getenv("NR_RT_GPUS")) {
         uint64_t x = 0;
@@ -303,6 +324,19 @@ int main(int argc, char** argv) {
             const char* v = need();
             if (!parse_u64(v, 0xFFFFFFFFull, &preview_every) || preview_every == 0)
                 die("invalid value '" + std::string(v) + "' for --preview-every");
+        } else if (a == "--adaptive-error") {
+            const char* v = need();
+            if (!parse_tolerance(v, &ad.rel_error)) die("invalid value '" + std::string(v) + "' for --adaptive-error");
+            adaptive = true;
+        } else if (a == "--adaptive-abs-error") {
+            const char* v = need();
+            if (!parse_tolerance(v, &ad.abs_error)) die("invalid value '" + std::string(v) + "' for --adaptive-abs-error");
+            adaptive_abs_set = true;
+        } else if (a == "--adaptive-min-samples") {
+            const char* v = need();
+            if (!parse_u64(v, 0xFFFFFFFFull, &adaptive_min))
+                die("invalid value '" + std::string(v) + "' for --adaptive-min-samples");
+            adaptive_min_set = true;
         }
         else if (a == "-W") { if (!set_camera("width", need())) die("invalid width"); }
         else if (a == "-H") { if (!set_camera("height", need())) die("invalid height"); }
@@ -319,6 +353,10 @@ int main(int argc, char** argv) {
     if (scene_path.empty()) die("missing <SCENE>");
     if (preview_every && gpus > 1)
         die("--preview-every renders on one GPU: it cannot be combined with --gpus " + std::to_string(gpus));
+    if ((adaptive_abs_set || adaptive_min_set) && !adaptive)
+        die(std::string(adaptive_abs_set ? "--adaptive-abs-error" : "--adaptive-min-samples") + " needs --adaptive-error");
+    if (adaptive && gpus > 1)
+        die("--adaptive-error renders on one GPU: it cannot be combined with --gpus " + std::to_string(gpus));
     auto ends = [&](const char* suf) {
         size_t n = std::strlen(suf);
         return output.size() >= n && output.compare(output.size() - n, n, suf) == 0;
@@ -373,26 +411,49 @@ int main(int argc, char** argv) {
         if (nrrt_render_multi(devs.data(), gpus, nrrt_host_scene_desc(hs), &cam, &opts, image.data(),
                               verbose ? on_progress : nullptr, nullptr, &st, msg, sizeof msg) != NRRT_OK)
             die(msg);
-    } else if (preview_every) {
+    } else if (preview_every || adaptive) {
         // progressive: each pass renders up to the next multiple of N samples (rounded up to a chunk boundary), then the
-        // image so far replaces the output file; the last pass completes the frame, which is nrrt_render's bit for bit
+        // image so far replaces the output file; the last pass completes the frame, which is nrrt_render's bit for bit.
+        // Adaptive: the passes render the pixels still active only, and end at doubling chunk counts unless
+        // --preview-every sets them; the frame is finished when no pixel is active.
         std::fclose(out);  // (opened above only for the create-new check: every image goes through replace_image)
         out = nullptr;
         nrrt_accum* acc = nullptr;
-        if (nrrt_accum_create(ctx, &cam, &opts, &acc) != NRRT_OK) die(nrrt_last_error(ctx));
         const uint32_t spp = cam.samples_per_pixel ? cam.samples_per_pixel : 1;
+        std::vector<uint32_t> starts(65);
+        const uint32_t n_chunks = nrrt_chunk_starts(spp, (uint64_t)cam.width * cam.height, starts.data(), 65);
+        uint32_t k = 1;  // chunk count the next adaptive pass ends on (without --preview-every)
+        if (adaptive) {
+            while (k < n_chunks && 8ull * starts[k] < spp) ++k;  // default: the first boundary at or above spp / 8
+            ad.min_samples = adaptive_min_set ? (uint32_t)adaptive_min : starts[k];
+            k = 1;
+            while (k < n_chunks && starts[k] < ad.min_samples) ++k;
+            if (nrrt_accum_create_adaptive(ctx, &cam, &opts, &ad, &acc) != NRRT_OK) die(nrrt_last_error(ctx));
+        } else if (nrrt_accum_create(ctx, &cam, &opts, &acc) != NRRT_OK) {
+            die(nrrt_last_error(ctx));
+        }
+        auto more = [&] { return adaptive ? nrrt_accum_active(acc) > 0 : nrrt_accum_samples(acc) < spp; };
         std::vector<uint8_t> preview(image.size());
         std::memset(&st, 0, sizeof st);
-        while (nrrt_accum_samples(acc) < spp) {
-            const uint64_t target = (nrrt_accum_samples(acc) / preview_every + 1) * preview_every;
+        while (more()) {
+            uint64_t target;
+            if (preview_every) {
+                target = (nrrt_accum_samples(acc) / preview_every + 1) * preview_every;
+            } else {
+                target = starts[std::min(k, n_chunks)];
+                k *= 2;
+            }
             nrrt_render_stats ps;
             if (nrrt_accum_render(acc, (uint32_t)std::min<uint64_t>(target, spp), &ps) != NRRT_OK) die(nrrt_last_error(ctx));
             st.paths += ps.paths, st.segments += ps.segments, st.launches += ps.launches, st.device_ms += ps.device_ms;
             const uint32_t done = nrrt_accum_samples(acc);
-            if (verbose)
-                std::fprintf(stderr, "pass: %u / %u samples  (%.3f s)\n", done, spp,
-                             std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count());
-            if (done < spp) {
+            const double secs = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
+            if (verbose && adaptive)
+                std::fprintf(stderr, "pass: %u / %u samples  %u pixels rendered  %u active  %llu segments  (%.3f s)\n", done,
+                             spp, ps.pixels, nrrt_accum_active(acc), (unsigned long long)ps.segments, secs);
+            else if (verbose)
+                std::fprintf(stderr, "pass: %u / %u samples  (%.3f s)\n", done, spp, secs);
+            if (preview_every && more()) {
                 if (nrrt_accum_image(acc, image.data(), 0) != NRRT_OK ||
                     nrrt_encode_rgb8(ctx, image.data(), cam.width, cam.height, gamma, 0, preview.data()) != NRRT_OK)
                     die(nrrt_last_error(ctx));

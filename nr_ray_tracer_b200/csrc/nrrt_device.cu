@@ -77,15 +77,18 @@ struct RenderParams {
     uint32_t chunk;          // samples of an equal-size work item (the first n_eq chunks of a pixel)
     uint32_t n_eq;           // equal chunks; they cover samples [0, n_eq * chunk)
     uint32_t n_chunks;       // work items per pixel = n_eq + the halving chunks over the remaining samples
-    uint32_t c0;             // first chunk of this launch: it renders chunks [c0, c0 + n_items / n_owned_pixels)
-    uint32_t n_items;        // n_owned_pixels * (chunks of this launch); items and partials are numbered from c0
+    uint32_t c0;             // first chunk of this launch: it renders chunks [c0, c0 + n_items / div_pixels.d)
+    uint32_t n_items;        // pixels of the launch * its chunks; items and partials are numbered from c0
     uint32_t long_end;       // item where this launch's equal chunks end (item_block_size)
     uint32_t n_slots;        // paths in flight
     uint32_t n_warps;        // warps that fetch work-item blocks (persistent kernels)
     uint32_t rank, world, rows_per_block;
-    FastDiv div_pixels, div_rows;  // by n_owned_pixels, rows_per_block
+    FastDiv div_pixels, div_rows;  // by the pixels of the launch (n_owned_pixels, or the active ones), rows_per_block
     FastDiv div_tile, div_strip, div_last;  // by tile_rows, by width * tile_rows (pixels of a full strip), by the rows of the last strip
     uint32_t full_strips;          // strips of tile_rows owned rows
+    // adaptive pass: the launch's pixels are active[0 .. div_pixels.d), owned-pixel indices in ascending order
+    // (null: every owned pixel, div_pixels.d = n_owned_pixels)
+    const uint32_t* active;
 };
 
 // owned pixel index -> (x, y) and the owned row j: rank owns row-blocks b with b % world == rank.
@@ -134,10 +137,23 @@ struct WorkItem {
 };
 // item -> pixel + sample range; returns the first sample.  The chunk c is absolute (the launch's item 0 is chunk c0's
 // first pixel), so a pixel's samples and their Philox counters do not depend on which launch renders them.
+// ACTIVE: an adaptive pass (P.active set), whose item's pixel is the po-th active one.  A compile-time flag, so that
+// the kernels of a plain render carry no trace of the list: tested at run time, the load is predicated rather than
+// branched around and the benchmark's one-shot render lost 0.5 % to it (measured on B200).
+template <bool ACTIVE = false>
 __host__ __device__ __forceinline__ uint32_t decode_item(const nrrt_camera& cam, const RenderParams& P, uint32_t item,
                                                          WorkItem& wi) {
-    uint32_t c = P.div_pixels.div(item), po = item - c * P.n_owned_pixels;
+    uint32_t c = P.div_pixels.div(item), po = item - c * (ACTIVE ? P.div_pixels.d : P.n_owned_pixels);
     c += P.c0;
+    if (ACTIVE) {
+#ifdef __CUDA_ARCH__
+        NRRT_CHECK(P.active && po < P.div_pixels.d, "active[] index");
+#endif
+        po = P.active[po];
+#ifdef __CUDA_ARCH__
+        NRRT_CHECK(po < P.n_owned_pixels, "active pixel is not an owned pixel");
+#endif
+    }
     uint32_t j;
     owned_pixel(cam, P, po, wi.x, wi.y, j);
     const uint32_t spp = cam.samples_per_pixel;
@@ -239,7 +255,7 @@ __device__ __forceinline__ bool path_step(const DevScene& S, const nrrt_camera& 
 
 // Megakernel variant: persistent threads, whole path state in registers.
 //   counters: [0]=segments [1]=paths [2..4]=node/exact/prim counts (COUNT) [5]=next work item
-template <bool COUNT>
+template <bool COUNT, bool ACTIVE>
 __global__ void __launch_bounds__(NRRT_BLOCK)
 k_render_mega(const __grid_constant__ DevScene S, const __grid_constant__ nrrt_camera cam,
               const __grid_constant__ RenderParams P, double* __restrict__ partials,
@@ -265,7 +281,7 @@ k_render_mega(const __grid_constant__ DevScene S, const __grid_constant__ nrrt_c
                     if (item >= P.n_items) {
                         running = false;
                     } else {
-                        smp.sample = decode_item(cam, P, item, wi);
+                        smp.sample = decode_item<ACTIVE>(cam, P, item, wi);
                         smp.pixel = wi.y * cam.width + wi.x;
                         sum = mk3(0.0, 0.0, 0.0);
                         have_item = true;
@@ -346,6 +362,176 @@ __global__ void k_resolve(const __grid_constant__ nrrt_camera cam, const __grid_
     d3 col = div3(s, samples);
     size_t ob = ((size_t)(packed ? j : y) * cam.width + x) * 3;  // packed: the rank's rows in ascending order
     out[ob] = (float)col.x, out[ob + 1] = (float)col.y, out[ob + 2] = (float)col.z;
+}
+
+// ---- adaptive sampling (include/nrrt.h).  The test is stated in f64 with every operation rounded on its own, so that
+// the host (nrrt_adaptive_converged, compiled with -ffp-contract=off) and a numpy restatement give the device's verdict.
+__host__ __device__ __forceinline__ double rn_add(double a, double b) {
+#ifdef __CUDA_ARCH__
+    return __dadd_rn(a, b);
+#else
+    return a + b;
+#endif
+}
+__host__ __device__ __forceinline__ double rn_sub(double a, double b) {
+#ifdef __CUDA_ARCH__
+    return __dsub_rn(a, b);
+#else
+    return a - b;
+#endif
+}
+__host__ __device__ __forceinline__ double rn_mul(double a, double b) {
+#ifdef __CUDA_ARCH__
+    return __dmul_rn(a, b);
+#else
+    return a * b;
+#endif
+}
+__host__ __device__ __forceinline__ double rn_div(double a, double b) {
+#ifdef __CUDA_ARCH__
+    return __ddiv_rn(a, b);
+#else
+    return a / b;
+#endif
+}
+// squared standard error of the mean of one channel, from the chunks as batch means (K >= 2; NaN propagates)
+__host__ __device__ __forceinline__ double adaptive_e2(double S, double Q, uint32_t N, uint32_t K) {
+    const double n = (double)N, x = rn_sub(Q, rn_div(rn_mul(S, S), n));
+    const double d = x < 0.0 ? 0.0 : x;  // rounding can leave Q - S*S/N slightly below zero
+    return rn_div(d, rn_mul((double)(K - 1), n));
+}
+__host__ __device__ __forceinline__ bool adaptive_converged(const double* S, const double* Q, uint32_t N, uint32_t K,
+                                                            const nrrt_adaptive_opts& T) {
+    if (K < 2 || N < T.min_samples || !(T.rel_error > 0.0 || T.abs_error > 0.0)) return false;
+    for (int ch = 0; ch < 3; ++ch) {
+        const double m = rn_div(S[ch], (double)N);
+        const double tol = rn_add(T.abs_error, rn_mul(T.rel_error, fabs(m)));
+        if (!(adaptive_e2(S[ch], Q[ch], N, K) <= rn_mul(tol, tol))) return false;
+    }
+    return true;
+}
+
+// Per-pixel state of an adaptive frame, owned rows packed ([j][x]; S and Q with 3 channels)
+struct AdaptiveState {
+    double* S;
+    double* Q;
+    uint32_t* N;
+    uint32_t* K;
+};
+
+// One thread per active pixel a of a pass over chunks [P.c0, c1): adds the pass's partials (item-indexed: chunk-local
+// c * n_active + a) to S and Q in chunk order, sets N and K, and writes keep[a] = the pixel stays active.  S gets the
+// additions k_resolve makes, so a pixel that runs every chunk ends on the one-shot sum.
+__global__ void k_resolve_adaptive(const __grid_constant__ nrrt_camera cam, const __grid_constant__ RenderParams P,
+                                   uint32_t n_active, const double* __restrict__ partials, AdaptiveState A,
+                                   const uint32_t* __restrict__ starts, uint32_t c1, nrrt_adaptive_opts T,
+                                   uint8_t* __restrict__ keep) {
+    const uint32_t a = blockIdx.x * blockDim.x + threadIdx.x;
+    if (a >= n_active) return;
+    const uint32_t po = P.active[a];
+    NRRT_CHECK(po < P.n_owned_pixels, "active pixel is not an owned pixel");
+    uint32_t x, y, j;
+    owned_pixel(cam, P, po, x, y, j);
+    const size_t pix = (size_t)j * cam.width + x;
+    NRRT_CHECK(pix < P.n_owned_pixels, "adaptive state index");
+    double s[3], q[3];
+    for (int ch = 0; ch < 3; ++ch) s[ch] = A.S[3 * pix + ch], q[ch] = A.Q[3 * pix + ch];
+    for (uint32_t c = P.c0; c < c1; ++c) {
+        const double n_c = (double)(starts[c + 1] - starts[c]);
+        const size_t b = ((size_t)(c - P.c0) * n_active + a) * 3;
+        for (int ch = 0; ch < 3; ++ch) {
+            const double p = partials[b + ch];
+            s[ch] = __dadd_rn(s[ch], p);
+            q[ch] = __dadd_rn(q[ch], __ddiv_rn(__dmul_rn(p, p), n_c));
+        }
+    }
+    for (int ch = 0; ch < 3; ++ch) A.S[3 * pix + ch] = s[ch], A.Q[3 * pix + ch] = q[ch];
+    A.N[pix] = starts[c1];
+    A.K[pix] = c1;
+    keep[a] = c1 < P.n_chunks && !adaptive_converged(s, q, starts[c1], c1, T);
+}
+
+// Ordered compaction of the active list: the kept entries of in[0 .. n), in their order, to out.  Deterministic (no
+// atomics), so the next pass's item order is a function of the retired set alone, and ascending stays ascending, so a
+// warp's block of items stays a compact tile of the remaining pixels.  (1) a count per block, (2) an exclusive scan of
+// the counts in one block, (3) each block scatters its kept entries from its offset on.
+#define NRRT_COMPACT_BLOCK 256
+__global__ void __launch_bounds__(NRRT_COMPACT_BLOCK) k_compact_count(const uint8_t* __restrict__ keep, uint32_t n,
+                                                                      uint32_t* __restrict__ counts) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    const int k = __syncthreads_count(i < n && keep[i]);
+    if (threadIdx.x == 0) counts[blockIdx.x] = (uint32_t)k;
+}
+__global__ void __launch_bounds__(1024) k_compact_scan(uint32_t* __restrict__ counts, uint32_t n_blocks,
+                                                       uint32_t* __restrict__ total) {
+    __shared__ uint32_t s[1024];
+    const uint32_t t = threadIdx.x, per = (n_blocks + 1023) / 1024;
+    const uint32_t b0 = min(t * per, n_blocks), b1 = min(b0 + per, n_blocks);
+    uint32_t mine = 0;
+    for (uint32_t b = b0; b < b1; ++b) mine += counts[b];
+    s[t] = mine;
+    __syncthreads();
+    for (uint32_t off = 1; off < 1024; off <<= 1) {  // inclusive scan over the threads' segment sums
+        const uint32_t v = t >= off ? s[t - off] : 0u;
+        __syncthreads();
+        s[t] += v;
+        __syncthreads();
+    }
+    uint32_t run = s[t] - mine;
+    for (uint32_t b = b0; b < b1; ++b) {
+        const uint32_t cnt = counts[b];
+        counts[b] = run;
+        run += cnt;
+    }
+    if (t == 1023) *total = s[t];
+}
+__global__ void __launch_bounds__(NRRT_COMPACT_BLOCK) k_compact_scatter(const uint32_t* __restrict__ in,
+                                                                        const uint8_t* __restrict__ keep, uint32_t n,
+                                                                        const uint32_t* __restrict__ offsets,
+                                                                        uint32_t* __restrict__ out) {
+    __shared__ uint32_t s_warp[NRRT_COMPACT_BLOCK / 32];
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const bool k = i < n && keep[i];
+    const uint32_t ballot = __ballot_sync(0xffffffffu, k);
+    if (lane == 0) s_warp[warp] = __popc(ballot);
+    __syncthreads();
+    uint32_t at = offsets[blockIdx.x];
+    for (uint32_t w = 0; w < warp; ++w) at += s_warp[w];
+    if (k) out[at + __popc(ballot & ((1u << lane) - 1u))] = in[i];
+}
+
+// Per-pixel outputs of an adaptive frame, one thread per owned pixel, laid out as k_resolve lays out the image
+// (packed: owned rows only).  IMAGE: S / N as f32; ERROR: sqrt(e2) per channel as f32, +inf where K < 2; SAMPLES: N.
+enum AdaptiveMap { AMAP_IMAGE, AMAP_ERROR, AMAP_SAMPLES };
+template <int WHAT>
+__global__ void k_adaptive_map(const __grid_constant__ nrrt_camera cam, const __grid_constant__ RenderParams P,
+                               AdaptiveState A, void* __restrict__ out, bool packed) {
+    const uint32_t po = blockIdx.x * blockDim.x + threadIdx.x;
+    if (po >= P.n_owned_pixels) return;
+    uint32_t x, y, j;
+    owned_pixel(cam, P, po, x, y, j);
+    const size_t pix = (size_t)j * cam.width + x;
+    NRRT_CHECK(pix < P.n_owned_pixels, "adaptive state index");
+    const size_t ob = (size_t)(packed ? j : y) * cam.width + x;
+    const uint32_t N = A.N[pix];
+    if (WHAT == AMAP_SAMPLES) {
+        static_cast<uint32_t*>(out)[ob] = N;
+        return;
+    }
+    float* o = static_cast<float*>(out) + 3 * ob;
+    for (int ch = 0; ch < 3; ++ch) {
+        if (WHAT == AMAP_IMAGE) {
+            o[ch] = (float)__ddiv_rn(A.S[3 * pix + ch], (double)N);
+        } else {
+            const uint32_t K = A.K[pix];
+            o[ch] = K < 2 ? __int_as_float(0x7f800000) : (float)__dsqrt_rn(adaptive_e2(A.S[3 * pix + ch], A.Q[3 * pix + ch], N, K));
+        }
+    }
+}
+
+__global__ void k_iota(uint32_t* __restrict__ out, uint32_t n) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) out[i] = i;
 }
 
 // output stage: gamma_correction (image.rs:53-57) + to_rgb8 (clamp, x255, round) — §8(f) N2
@@ -509,7 +695,7 @@ k_render_fused(const __grid_constant__ DevScene S, const __grid_constant__ nrrt_
                     state = RETIRED;
                 } else {
                     WorkItem wi;
-                    smp.sample = decode_item(cam, P, s_item, wi);
+                    smp.sample = decode_item<(F & NRRT_F_ACTIVE) != 0>(cam, P, s_item, wi);
                     smp.pixel = wi.y * cam.width + wi.x;
                     s_px = wi.x, s_py = wi.y, s_end = wi.sample_end;
                     st[9 * NRRT_BLOCK] = 0.0, st[10 * NRRT_BLOCK] = 0.0, st[11 * NRRT_BLOCK] = 0.0;
@@ -622,6 +808,7 @@ __device__ __forceinline__ uint32_t queue_slot(const uint32_t* q, uint32_t n, ui
 }
 
 // ray generation for the initial items
+template <bool ACTIVE>
 __global__ void __launch_bounds__(NRRT_BLOCK)
 k_wf_init(const __grid_constant__ nrrt_camera cam, const __grid_constant__ RenderParams P,
           const __grid_constant__ WfState W) {
@@ -638,7 +825,7 @@ k_wf_init(const __grid_constant__ nrrt_camera cam, const __grid_constant__ Rende
     if (w >= P.n_slots) return;
     uint32_t n = P.n_slots;
     WorkItem wi;
-    uint32_t first = decode_item(cam, P, w, wi);
+    uint32_t first = decode_item<ACTIVE>(cam, P, w, wi);
     Sampler smp{P.key, wi.y * cam.width + wi.x, first};
     d3 o, d;
     double tm;
@@ -736,7 +923,7 @@ k_wf_shade(const __grid_constant__ DevScene S, const __grid_constant__ nrrt_came
         L = mk3(0.0, 0.0, 0.0);
         bounce = W.bounce[slot];
         item = W.item[slot];
-        decode_item(cam, P, item, wi);
+        decode_item<(F & NRRT_F_ACTIVE) != 0>(cam, P, item, wi);
         smp.pixel = wi.y * cam.width + wi.x;
         smp.sample = W.sample[slot];
         HitId h;
@@ -794,7 +981,7 @@ k_wf_shade(const __grid_constant__ DevScene S, const __grid_constant__ nrrt_came
         if (need_item) {
             item = base + __popc(need & ((1u << lane_id) - 1u));
             if (item < P.n_items) {
-                smp.sample = decode_item(cam, P, item, wi);
+                smp.sample = decode_item<(F & NRRT_F_ACTIVE) != 0>(cam, P, item, wi);
                 smp.pixel = wi.y * cam.width + wi.x;
                 W.item[slot] = item;
                 new_path = true;
@@ -1377,11 +1564,15 @@ static void launch_extend(nrrt_ctx* ctx, unsigned blocks, size_t smem, const WfS
 static void launch_shade(nrrt_ctx* ctx, unsigned blocks, const nrrt_camera& c, const RenderParams& P, const WfState& Wf,
                          uint32_t qin) {
     switch (ctx->features) {
-        case NRRT_F_CORNELL: k_wf_shade<NRRT_F_CORNELL><<<blocks, NRRT_BLOCK, 0, ctx->stream>>>(ctx->dev, c, P, Wf, qin); break;
-        case NRRT_F_BALLS: k_wf_shade<NRRT_F_BALLS><<<blocks, NRRT_BLOCK, 0, ctx->stream>>>(ctx->dev, c, P, Wf, qin); break;
-        case NRRT_F_BALLS_TEX: k_wf_shade<NRRT_F_BALLS_TEX><<<blocks, NRRT_BLOCK, 0, ctx->stream>>>(ctx->dev, c, P, Wf, qin); break;
-        case NRRT_F_GENERAL: k_wf_shade<NRRT_F_GENERAL><<<blocks, NRRT_BLOCK, 0, ctx->stream>>>(ctx->dev, c, P, Wf, qin); break;
-        default: k_wf_shade<NRRT_F_ALL><<<blocks, NRRT_BLOCK, 0, ctx->stream>>>(ctx->dev, c, P, Wf, qin); break;
+#define NRRT_SHADE_CASE(FEAT)                                                                                   \
+    if (P.active) k_wf_shade<FEAT | NRRT_F_ACTIVE><<<blocks, NRRT_BLOCK, 0, ctx->stream>>>(ctx->dev, c, P, Wf, qin); \
+    else k_wf_shade<FEAT><<<blocks, NRRT_BLOCK, 0, ctx->stream>>>(ctx->dev, c, P, Wf, qin);
+        case NRRT_F_CORNELL: NRRT_SHADE_CASE(NRRT_F_CORNELL) break;
+        case NRRT_F_BALLS: NRRT_SHADE_CASE(NRRT_F_BALLS) break;
+        case NRRT_F_BALLS_TEX: NRRT_SHADE_CASE(NRRT_F_BALLS_TEX) break;
+        case NRRT_F_GENERAL: NRRT_SHADE_CASE(NRRT_F_GENERAL) break;
+        default: NRRT_SHADE_CASE(NRRT_F_ALL) break;
+#undef NRRT_SHADE_CASE
     }
 }
 
@@ -1393,11 +1584,17 @@ static cudaError_t launch_fused(nrrt_ctx* ctx, unsigned blocks, const nrrt_camer
     e = cudaFuncSetAttribute(k_render_fused<FEAT, MB, SPEC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);  \
     if (e == cudaSuccess)                                                                                              \
         k_render_fused<FEAT, MB, SPEC><<<blocks, NRRT_BLOCK, smem, ctx->stream>>>(ctx->dev, c, P, partials, ctx->d_counters);
-#define NRRT_FUSED_CASE(FEAT, MB)                                                                                      \
+#define NRRT_FUSED_SPEC(FEAT, MB)                                                                                      \
     if (ctx->speculate) {                                                                                              \
         NRRT_FUSED_LAUNCH(FEAT, MB, true)                                                                              \
     } else {                                                                                                           \
         NRRT_FUSED_LAUNCH(FEAT, MB, false)                                                                             \
+    }
+#define NRRT_FUSED_CASE(FEAT, MB)                                                                                      \
+    if (P.active) {                                                                                                    \
+        NRRT_FUSED_SPEC(FEAT | NRRT_F_ACTIVE, MB)                                                                      \
+    } else {                                                                                                           \
+        NRRT_FUSED_SPEC(FEAT, MB)                                                                                      \
     }
     switch (ctx->features) {
         case NRRT_F_CORNELL: NRRT_FUSED_CASE(NRRT_F_CORNELL, NRRT_FUSED_BLOCKS_PER_SM) break;
@@ -1407,6 +1604,7 @@ static cudaError_t launch_fused(nrrt_ctx* ctx, unsigned blocks, const nrrt_camer
         default: NRRT_FUSED_CASE(NRRT_F_ALL, NRRT_FUSED_BLOCKS_PER_SM) break;
     }
 #undef NRRT_FUSED_CASE
+#undef NRRT_FUSED_SPEC
 #undef NRRT_FUSED_LAUNCH
     return e;
 }
@@ -1458,8 +1656,11 @@ static PoolPlan pool_plan_f(const nrrt_ctx* ctx) {
     best.slots = (uint64_t)ctx->sms * best_warps * NRRT_POOL_NS;
     return best;
 }
-static PoolPlan pool_plan(const nrrt_ctx* ctx, bool lite) {
-#define NRRT_POOL_PLAN(FEAT) return lite ? pool_plan_f<FEAT, true>(ctx) : pool_plan_f<FEAT, false>(ctx);
+// (active: the instantiations of an adaptive pass, NRRT_F_ACTIVE)
+static PoolPlan pool_plan(const nrrt_ctx* ctx, bool lite, bool active) {
+#define NRRT_POOL_PLAN(FEAT)                                                                                     \
+    if (active) return lite ? pool_plan_f<FEAT | NRRT_F_ACTIVE, true>(ctx) : pool_plan_f<FEAT | NRRT_F_ACTIVE, false>(ctx); \
+    return lite ? pool_plan_f<FEAT, true>(ctx) : pool_plan_f<FEAT, false>(ctx);
     switch (ctx->features) {
         case NRRT_F_CORNELL: NRRT_POOL_PLAN(NRRT_F_CORNELL)
         case NRRT_F_BALLS: NRRT_POOL_PLAN(NRRT_F_BALLS)
@@ -1485,11 +1686,17 @@ static cudaError_t launch_pool(nrrt_ctx* ctx, const PoolPlan& pl, const nrrt_cam
     if (e == cudaSuccess)                                                                                                 \
         k_render_pool<FEAT, NRRT_POOL_NS, LITE><<<blocks, pl.warps_per_block * 32, pl.smem, ctx->stream>>>(               \
             ctx->dev, c, P, partials, ctx->d_counters, pl.cap, cold, cold_slots);
-#define NRRT_POOL_LAUNCH(FEAT)                                                                                            \
+#define NRRT_POOL_LITE(FEAT)                                                                                              \
     if (pl.lite) {                                                                                                        \
         NRRT_POOL_LAUNCH_L(FEAT, true)                                                                                    \
     } else {                                                                                                              \
         NRRT_POOL_LAUNCH_L(FEAT, false)                                                                                   \
+    }
+#define NRRT_POOL_LAUNCH(FEAT)                                                                                            \
+    if (P.active) {                                                                                                       \
+        NRRT_POOL_LITE(FEAT | NRRT_F_ACTIVE)                                                                              \
+    } else {                                                                                                              \
+        NRRT_POOL_LITE(FEAT)                                                                                              \
     }
     switch (ctx->features) {
         case NRRT_F_CORNELL: NRRT_POOL_LAUNCH(NRRT_F_CORNELL) break;
@@ -1499,6 +1706,7 @@ static cudaError_t launch_pool(nrrt_ctx* ctx, const PoolPlan& pl, const nrrt_cam
         default: NRRT_POOL_LAUNCH(NRRT_F_ALL) break;
     }
 #undef NRRT_POOL_LAUNCH_L
+#undef NRRT_POOL_LITE
 #undef NRRT_POOL_LAUNCH
     return e;
 }
@@ -1626,12 +1834,17 @@ static uint32_t owned_rows(uint32_t H, uint32_t rank, uint32_t world, uint32_t R
 
 // Partition and work-item fields of RenderParams (everything decode_item / owned_pixel / item_block_size read, bar the
 // slot counts) of a launch over chunks [c0, c1) (c1 clamped to the pixel's chunks): shared by the renders and
-// nrrt_work_items / nrrt_pass_items.  Returns nullptr or the reason it cannot be done.
+// nrrt_work_items / nrrt_pass_items.  With `active` (an adaptive pass) the launch covers the n_active owned pixels it
+// lists instead of every owned pixel.  Returns nullptr or the reason it cannot be done.
 static const char* work_item_params(RenderParams& P, uint32_t W, uint32_t H, uint32_t spp, uint32_t rank, uint32_t world,
-                                    uint32_t rows_per_block, uint32_t c0 = 0, uint32_t c1 = 0xFFFFFFFFu) {
+                                    uint32_t rows_per_block, uint32_t c0 = 0, uint32_t c1 = 0xFFFFFFFFu,
+                                    const uint32_t* active = nullptr, uint32_t n_active = 0) {
     const uint64_t total_pixels = (uint64_t)W * H;
     P.rank = rank, P.world = world, P.rows_per_block = rows_per_block;
     P.n_owned_pixels = owned_rows(H, rank, world, rows_per_block) * W;
+    P.active = active;
+    const uint32_t n_pixels = active ? n_active : P.n_owned_pixels;  // pixels of each chunk of the launch
+    if (n_pixels > P.n_owned_pixels) return "internal error: more active pixels than owned ones";
     // Work items of a pixel.  They fix the order in which its samples are summed, so they may depend only on what
     // every rank of every partition agrees on — spp and the size of the WHOLE image — never on slots, rank or world:
     // the image is then bit-identical for every slot count and GPU count.  Items are numbered chunk-major (every
@@ -1654,13 +1867,13 @@ static const char* work_item_params(RenderParams& P, uint32_t W, uint32_t H, uin
     chunk_schedule(spp, total_pixels, P.chunk, P.n_eq, P.n_chunks);
     c1 = std::min(c1, P.n_chunks);
     if (c0 > c1) return "chunk range past the last chunk";
-    const uint64_t n_items64 = (uint64_t)P.n_owned_pixels * (c1 - c0);
+    const uint64_t n_items64 = (uint64_t)n_pixels * (c1 - c0);
     if (n_items64 > 0xFFFFFFF0ull) return "too many work items";
     P.c0 = c0;
     P.n_items = (uint32_t)n_items64;
-    P.long_end = (std::min(std::max(P.n_eq, c0), c1) - c0) * P.n_owned_pixels;  // (fits: n_items does)
+    P.long_end = (std::min(std::max(P.n_eq, c0), c1) - c0) * n_pixels;  // (fits: n_items does)
     P.n_slots = P.n_warps = 0;
-    P.div_pixels = FastDiv::make(P.n_owned_pixels);
+    P.div_pixels = FastDiv::make(n_pixels);
     P.div_rows = FastDiv::make(rows_per_block);
     {
         const uint32_t rows = P.n_owned_pixels / W;
@@ -1673,8 +1886,8 @@ static const char* work_item_params(RenderParams& P, uint32_t W, uint32_t H, uin
         P.full_strips = rows / tile_rows;
         P.div_last = FastDiv::make(std::max<uint32_t>(rows % tile_rows, 1));
     }
-    for (uint32_t probe : {0u, 1u, W - 1, W, W + 1, P.n_owned_pixels - 1, P.n_owned_pixels, P.n_items - 1, 0x7fffffffu,
-                           0xfffffff0u}) {  // the multiply-shift must agree with '/' (cheap self-check)
+    for (uint32_t probe : {0u, 1u, W - 1, W, W + 1, P.n_owned_pixels - 1, P.n_owned_pixels, n_pixels - 1, n_pixels,
+                           P.n_items - 1, 0x7fffffffu, 0xfffffff0u}) {  // the multiply-shift must agree with '/' (cheap self-check)
         if (P.div_pixels.div(probe) != probe / P.div_pixels.d || P.div_strip.div(probe) != probe / P.div_strip.d ||
             P.div_rows.div(probe) != probe / P.div_rows.d || P.div_last.div(probe) != probe / P.div_last.d ||
             P.div_tile.div(probe) != probe / P.div_tile.d)
@@ -1683,11 +1896,12 @@ static const char* work_item_params(RenderParams& P, uint32_t W, uint32_t H, uin
     return nullptr;
 }
 
-// Work items [first, first + n) of one rank's launch over chunks [c0, c1), decoded by the very functions the kernels
-// use: 4 values per item (x, y, first sample, one past the last sample).  Returns the number of items of that launch, 0
-// if the arguments are not ones the renders would take.
-uint32_t nrrt_pass_items(uint32_t width, uint32_t height, uint32_t samples_per_pixel, uint32_t rank, uint32_t world,
-                         uint32_t rows_per_block, uint32_t c0, uint32_t c1, uint32_t first, uint32_t n, uint32_t* out) {
+// Work items [first, first + n) of one rank's launch over chunks [c0, c1) (and the active pixels, see
+// work_item_params), decoded by the very functions the kernels use: 4 values per item (x, y, first sample, one past the
+// last sample).  Returns the number of items of that launch, 0 if the arguments are not ones the renders would take.
+static uint32_t decode_pass(uint32_t width, uint32_t height, uint32_t samples_per_pixel, uint32_t rank, uint32_t world,
+                            uint32_t rows_per_block, uint32_t c0, uint32_t c1, const uint32_t* active, uint32_t n_active,
+                            uint32_t first, uint32_t n, uint32_t* out) {
     if (width == 0 || height == 0 || (uint64_t)width * height > 0x7FFFFFFFull) return 0;
     if (world == 0) world = 1;
     if (rank >= world) return 0;
@@ -1697,13 +1911,19 @@ uint32_t nrrt_pass_items(uint32_t width, uint32_t height, uint32_t samples_per_p
     nrrt_camera cam;
     std::memset(&cam, 0, sizeof cam);
     cam.width = width, cam.height = height, cam.samples_per_pixel = std::max<uint32_t>(samples_per_pixel, 1);
-    if (work_item_params(P, width, height, cam.samples_per_pixel, rank, world, rows_per_block, c0, c1)) return 0;
+    if (work_item_params(P, width, height, cam.samples_per_pixel, rank, world, rows_per_block, c0, c1, active, n_active))
+        return 0;
     for (uint32_t i = 0; out && i < n && (uint64_t)first + i < P.n_items; ++i) {
         WorkItem wi;
-        const uint32_t s0 = decode_item(cam, P, first + i, wi);
+        const uint32_t s0 = active ? decode_item<true>(cam, P, first + i, wi) : decode_item<false>(cam, P, first + i, wi);
         out[4 * i + 0] = wi.x, out[4 * i + 1] = wi.y, out[4 * i + 2] = s0, out[4 * i + 3] = wi.sample_end;
     }
     return P.n_items;
+}
+
+uint32_t nrrt_pass_items(uint32_t width, uint32_t height, uint32_t samples_per_pixel, uint32_t rank, uint32_t world,
+                         uint32_t rows_per_block, uint32_t c0, uint32_t c1, uint32_t first, uint32_t n, uint32_t* out) {
+    return decode_pass(width, height, samples_per_pixel, rank, world, rows_per_block, c0, c1, nullptr, 0, first, n, out);
 }
 
 uint32_t nrrt_work_items(uint32_t width, uint32_t height, uint32_t samples_per_pixel, uint32_t rank, uint32_t world,
@@ -1711,17 +1931,53 @@ uint32_t nrrt_work_items(uint32_t width, uint32_t height, uint32_t samples_per_p
     return nrrt_pass_items(width, height, samples_per_pixel, rank, world, rows_per_block, 0, 0xFFFFFFFFu, first, n, out);
 }
 
+// The active list of an adaptive pass: strictly ascending owned-pixel indices, each below n_owned
+static bool active_list_ok(const uint32_t* active, uint32_t n_active, uint32_t n_owned) {
+    if (n_active && !active) return false;
+    for (uint32_t i = 0; i < n_active; ++i)
+        if (active[i] >= n_owned || (i && active[i] <= active[i - 1])) return false;
+    return true;
+}
+
+uint32_t nrrt_pass_items_active(uint32_t width, uint32_t height, uint32_t samples_per_pixel, uint32_t rank,
+                                uint32_t world, uint32_t rows_per_block, uint32_t c0, uint32_t c1,
+                                const uint32_t* active, uint32_t n_active, uint32_t first, uint32_t n, uint32_t* out) {
+    const uint32_t wd = world ? world : 1;
+    if (width == 0 || height == 0 || (uint64_t)width * height > 0x7FFFFFFFull || rank >= wd) return 0;
+    if (!active_list_ok(active, n_active, owned_rows(height, rank, wd, rows_per_block ? rows_per_block : 8) * width))
+        return 0;
+    static const uint32_t none = 0;  // a non-null list for n_active = 0: a pass over no pixel, not over all of them
+    return decode_pass(width, height, samples_per_pixel, rank, world, rows_per_block, c0, c1, active ? active : &none,
+                       n_active, first, n, out);
+}
+
+// An adaptive pass of render_chunks: the pixels it renders, and what k_resolve_adaptive and the compaction need
+struct AdaptivePass {
+    const uint32_t* active;  // n_active ascending owned-pixel indices (device)
+    uint32_t n_active;
+    AdaptiveState state;
+    const uint32_t* starts;  // nrrt_chunk_starts of the frame (device)
+    nrrt_adaptive_opts test;
+    uint8_t* keep;           // [n_active]
+    uint32_t* block_counts;  // [blocks of NRRT_COMPACT_BLOCK over n_active]
+    uint32_t* next_active;   // receives the pixels still active after the pass, in order ...
+    uint32_t* n_next;        // ... and their count
+};
+
 // Renders chunks [c0, c1) of every pixel rank o.rank owns (o.world >= 1, o.rows_per_block >= 1) into the scratch
 // partials and resolves them (k_resolve) onto acc (may be null) and, divided by `samples`, into the image *fb (may be
 // null; with fb_scratch a full-size image is carved in the scratch and returned in *fb): the body of nrrt_render (all
-// chunks) and of nrrt_accum_render (a pass).  Picks the design, carves the scratch, launches, and fills stats.
+// chunks) and of nrrt_accum_render (a pass).  An adaptive pass (ad) renders the active pixels only and resolves them
+// with k_resolve_adaptive instead, then compacts the active list.  Picks the design, carves the scratch, launches, and
+// fills stats.
 static int render_chunks(nrrt_ctx* ctx, const nrrt_camera& c, nrrt_render_opts o, uint32_t c0, uint32_t c1, double* acc,
                          double samples, float** fb, bool fb_scratch, bool packed, nrrt_progress_fn progress, void* user,
-                         nrrt_render_stats* stats, const char* who) {
+                         nrrt_render_stats* stats, const char* who, const AdaptivePass* ad = nullptr) {
     const uint32_t W = c.width, H = c.height;
     RenderParams P;
     P.key = make_uint2((uint32_t)o.seed, (uint32_t)(o.seed >> 32));
-    if (const char* why = work_item_params(P, W, H, c.samples_per_pixel, o.rank, o.world, o.rows_per_block, c0, c1)) {
+    if (const char* why = work_item_params(P, W, H, c.samples_per_pixel, o.rank, o.world, o.rows_per_block, c0, c1,
+                                           ad ? ad->active : nullptr, ad ? ad->n_active : 0)) {
         ctx->err = std::string(who) + ": " + why;
         return std::strstr(why, "internal") ? NRRT_ERR_INVALID : NRRT_ERR_LIMIT;
     }
@@ -1752,7 +2008,7 @@ static int render_chunks(nrrt_ctx* ctx, const nrrt_camera& c, nrrt_render_opts o
         // small scenes (binary nodes on the device): the two-stage variant
         bool lite = ctx->has_binary;
         if (const char* e = std::getenv("NRRT_POOL_LITE")) lite = std::atoi(e) != 0 && ctx->has_binary;  // developer override
-        plan = pool_plan(ctx, lite);
+        plan = pool_plan(ctx, lite, P.active != nullptr);
         if (plan.warps_per_block == 0) {
             ctx->err = "pooled kernel: the slot pool does not fit in shared memory";
             return NRRT_ERR_LIMIT;
@@ -1833,10 +2089,14 @@ static int render_chunks(nrrt_ctx* ctx, const nrrt_camera& c, nrrt_render_opts o
         CK(cudaGetLastError());
         ++launches;
     } else if (!wavefront) {
-        if (counting)
-            k_render_mega<true><<<work_blocks, NRRT_BLOCK, smem, ctx->stream>>>(ctx->dev, c, P, d_part, ctx->d_counters);
+        if (counting && P.active)
+            k_render_mega<true, true><<<work_blocks, NRRT_BLOCK, smem, ctx->stream>>>(ctx->dev, c, P, d_part, ctx->d_counters);
+        else if (counting)
+            k_render_mega<true, false><<<work_blocks, NRRT_BLOCK, smem, ctx->stream>>>(ctx->dev, c, P, d_part, ctx->d_counters);
+        else if (P.active)
+            k_render_mega<false, true><<<work_blocks, NRRT_BLOCK, smem, ctx->stream>>>(ctx->dev, c, P, d_part, ctx->d_counters);
         else
-            k_render_mega<false><<<work_blocks, NRRT_BLOCK, smem, ctx->stream>>>(ctx->dev, c, P, d_part, ctx->d_counters);
+            k_render_mega<false, false><<<work_blocks, NRRT_BLOCK, smem, ctx->stream>>>(ctx->dev, c, P, d_part, ctx->d_counters);
         CK(cudaGetLastError());
         ++launches;
     } else {
@@ -1857,7 +2117,8 @@ static int render_chunks(nrrt_ctx* ctx, const nrrt_camera& c, nrrt_render_opts o
         Wf.cursor = Wf.count + 4;
         Wf.partials = d_part;
         Wf.counters = ctx->d_counters;
-        k_wf_init<<<work_blocks, NRRT_BLOCK, 0, ctx->stream>>>(c, P, Wf);
+        if (P.active) k_wf_init<true><<<work_blocks, NRRT_BLOCK, 0, ctx->stream>>>(c, P, Wf);
+        else k_wf_init<false><<<work_blocks, NRRT_BLOCK, 0, ctx->stream>>>(c, P, Wf);
         CK(cudaGetLastError());
         ++launches;
         // the queue length lives on the device; the host polls it through a pinned ring without stalling
@@ -1931,7 +2192,20 @@ static int render_chunks(nrrt_ctx* ctx, const nrrt_camera& c, nrrt_render_opts o
         }
         if (!timing.empty()) extend_ms = sampled / (double)timing.size() * (double)extend_launches;
     }
-    if (P.n_owned_pixels) {
+    if (ad) {
+        if (ad->n_active) {
+            const uint32_t blocks = (ad->n_active + NRRT_COMPACT_BLOCK - 1) / NRRT_COMPACT_BLOCK;
+            k_resolve_adaptive<<<blocks, NRRT_COMPACT_BLOCK, 0, ctx->stream>>>(c, P, ad->n_active, d_part, ad->state,
+                                                                               ad->starts, P.c0 + P.n_items / ad->n_active,
+                                                                               ad->test, ad->keep);
+            k_compact_count<<<blocks, NRRT_COMPACT_BLOCK, 0, ctx->stream>>>(ad->keep, ad->n_active, ad->block_counts);
+            k_compact_scan<<<1, 1024, 0, ctx->stream>>>(ad->block_counts, blocks, ad->n_next);
+            k_compact_scatter<<<blocks, NRRT_COMPACT_BLOCK, 0, ctx->stream>>>(ad->active, ad->keep, ad->n_active,
+                                                                              ad->block_counts, ad->next_active);
+            CK(cudaGetLastError());
+            launches += 4;
+        }
+    } else if (P.n_owned_pixels) {
         k_resolve<<<(P.n_owned_pixels + 255) / 256, 256, 0, ctx->stream>>>(c, P, d_part, acc, samples, d_fb, packed);
         CK(cudaGetLastError());
         ++launches;
@@ -1968,7 +2242,7 @@ static int render_chunks(nrrt_ctx* ctx, const nrrt_camera& c, nrrt_render_opts o
         stats->device_ms = ms;
         stats->extend_ms = wavefront ? extend_ms : ms;
         stats->extend_launches = wavefront ? extend_launches : (launches ? 1 : 0);
-        stats->pixels = P.n_owned_pixels;
+        stats->pixels = ad ? ad->n_active : P.n_owned_pixels;
         stats->mode = counting ? (uint32_t)NRRT_MODE_MEGAKERNEL : o.mode;
         stats->node_visits = hc[2];
         stats->box_exact = hc[3];
@@ -1979,11 +2253,12 @@ static int render_chunks(nrrt_ctx* ctx, const nrrt_camera& c, nrrt_render_opts o
     return NRRT_OK;
 }
 
-// The rows rank o.rank owns, from the device image d_fb (full-size, or packed) to the caller's host buffer.
+// The rows rank o.rank owns, from the device image d_fb (full-size, or packed; px_bytes per pixel) to the caller's host
+// buffer.
 static int copy_owned_rows(nrrt_ctx* ctx, const nrrt_render_opts& o, uint32_t W, uint32_t H, bool packed,
-                           const float* d_fb, float* out_rgb) {
+                           const void* d_fb, void* out_rgb, size_t px_bytes = 3 * sizeof(float)) {
     const uint32_t R = o.rows_per_block;
-    const size_t row_bytes = (size_t)W * 3 * sizeof(float);
+    const size_t row_bytes = (size_t)W * px_bytes;
     if (packed) {
         const size_t rows = owned_rows(H, o.rank, o.world, R);
         if (rows) CK(cudaMemcpyAsync(out_rgb, d_fb, rows * row_bytes, cudaMemcpyDeviceToHost, ctx->stream));
@@ -2065,6 +2340,18 @@ struct nrrt_accum {
     uint32_t chunks_done = 0;
     size_t n_sums = 0;              // 3 x owned pixels
     double* d_sum = nullptr;        // running per-pixel sums, owned rows packed: [j][x][3]
+    // adaptive frames only (nrrt_accum_create_adaptive)
+    bool adaptive = false;
+    nrrt_adaptive_opts test;
+    uint32_t n_active = 0;          // pixels still active (every owned pixel before the first pass)
+    uint32_t cur = 0;               // d_active[cur] is the active list; a pass compacts it into the other one
+    void* d_ad = nullptr;           // one allocation for everything below
+    AdaptiveState st;               // S = d_sum; Q, N, K
+    uint32_t* d_active[2] = {nullptr, nullptr};
+    uint8_t* d_keep = nullptr;      // [owned pixels]: k_resolve_adaptive's verdicts
+    uint32_t* d_blocks = nullptr;   // compaction block counts
+    uint32_t* d_n_next = nullptr;   // compaction result count
+    uint32_t* d_starts = nullptr;   // starts on the device
 };
 
 // the accumulator's context is usable and still holds the scene the accumulator was created for
@@ -2079,24 +2366,37 @@ static int accum_check(const nrrt_accum* a, const char* who) {
     return NRRT_OK;
 }
 
-int nrrt_accum_create(nrrt_ctx* ctx, const nrrt_camera* cam, const nrrt_render_opts* opts_in, nrrt_accum** out) {
+static void accum_release(nrrt_accum* a) {
+    if (a->d_sum) cudaFree(a->d_sum);
+    if (a->d_ad) cudaFree(a->d_ad);
+    delete a;
+}
+
+// the body of nrrt_accum_create and nrrt_accum_create_adaptive (test: null for a plain progressive frame)
+static int accum_create(nrrt_ctx* ctx, const nrrt_camera* cam, const nrrt_render_opts* opts_in,
+                        const nrrt_adaptive_opts* test, nrrt_accum** out, const char* who) {
     if (!ctx || !out) return NRRT_ERR_INVALID;
     *out = nullptr;
     if (!ctx->has_scene) {
-        ctx->err = "nrrt_accum_create before nrrt_scene_upload";
+        ctx->err = std::string(who) + " before nrrt_scene_upload";
         return NRRT_ERR_NO_SCENE;
     }
     if (!cam || cam->width == 0 || cam->height == 0) {
-        ctx->err = "nrrt_accum_create: bad camera";
+        ctx->err = std::string(who) + ": bad camera";
         return NRRT_ERR_INVALID;
     }
     nrrt_render_opts o;
     if (const char* why = default_opts(opts_in, o)) {
-        ctx->err = std::string("nrrt_accum_create: ") + why;
+        ctx->err = std::string(who) + ": " + why;
         return NRRT_ERR_INVALID;
     }
     if (o.mode > NRRT_MODE_AUTO) {
-        ctx->err = "nrrt_accum_create: unknown mode";
+        ctx->err = std::string(who) + ": unknown mode";
+        return NRRT_ERR_INVALID;
+    }
+    if (test && !(std::isfinite(test->rel_error) && test->rel_error >= 0.0 && std::isfinite(test->abs_error) &&
+                  test->abs_error >= 0.0)) {
+        ctx->err = std::string(who) + ": rel_error and abs_error must be finite and >= 0";
         return NRRT_ERR_INVALID;
     }
     o.flags &= NRRT_RENDER_COUNT;  // the output flags belong to nrrt_accum_image
@@ -2119,14 +2419,58 @@ int nrrt_accum_create(nrrt_ctx* ctx, const nrrt_camera* cam, const nrrt_render_o
     const size_t bytes = std::max<size_t>(a->n_sums, 1) * sizeof(double);
     cudaError_t e = cudaMalloc((void**)&a->d_sum, bytes);
     if (e == cudaSuccess) e = cudaMemsetAsync(a->d_sum, 0, bytes, ctx->stream);
+    if (e == cudaSuccess && test) {
+        a->adaptive = true;
+        a->test = *test;
+        const size_t n = std::max<size_t>(a->n_sums / 3, 1), blocks = (n + NRRT_COMPACT_BLOCK - 1) / NRRT_COMPACT_BLOCK;
+        size_t off = 0;
+        auto carve = [&](size_t b) {
+            size_t at = off;
+            off += (b + 255) & ~(size_t)255;
+            return at;
+        };
+        const size_t o_q = carve(n * 3 * sizeof(double)), o_n = carve(n * 4), o_k = carve(n * 4), o_a0 = carve(n * 4),
+                     o_a1 = carve(n * 4), o_keep = carve(n), o_blk = carve(blocks * 4), o_cnt = carve(4),
+                     o_st = carve(a->starts.size() * 4);
+        e = cudaMalloc(&a->d_ad, off);
+        if (e == cudaSuccess) e = cudaMemsetAsync(a->d_ad, 0, off, ctx->stream);
+        if (e == cudaSuccess) {
+            char* base = (char*)a->d_ad;
+            a->st = AdaptiveState{a->d_sum, (double*)(base + o_q), (uint32_t*)(base + o_n), (uint32_t*)(base + o_k)};
+            a->d_active[0] = (uint32_t*)(base + o_a0), a->d_active[1] = (uint32_t*)(base + o_a1);
+            a->d_keep = (uint8_t*)(base + o_keep);
+            a->d_blocks = (uint32_t*)(base + o_blk);
+            a->d_n_next = (uint32_t*)(base + o_cnt);
+            a->d_starts = (uint32_t*)(base + o_st);
+            a->n_active = (uint32_t)(a->n_sums / 3);
+            e = cudaMemcpyAsync(a->d_starts, a->starts.data(), a->starts.size() * 4, cudaMemcpyHostToDevice, ctx->stream);
+            if (e == cudaSuccess && a->n_active) {
+                k_iota<<<(a->n_active + 255) / 256, 256, 0, ctx->stream>>>(a->d_active[0], a->n_active);
+                e = cudaGetLastError();
+            }
+        }
+    }
     if (e != cudaSuccess) {
-        ctx->err = std::string("nrrt_accum_create: ") + cudaGetErrorString(e);
-        if (a->d_sum) cudaFree(a->d_sum);
-        delete a;
+        ctx->err = std::string(who) + ": " + cudaGetErrorString(e);
+        accum_release(a);
         return NRRT_ERR_CUDA;
     }
     *out = a;
     return NRRT_OK;
+}
+
+int nrrt_accum_create(nrrt_ctx* ctx, const nrrt_camera* cam, const nrrt_render_opts* opts_in, nrrt_accum** out) {
+    return accum_create(ctx, cam, opts_in, nullptr, out, "nrrt_accum_create");
+}
+
+int nrrt_accum_create_adaptive(nrrt_ctx* ctx, const nrrt_camera* cam, const nrrt_render_opts* opts_in,
+                               const nrrt_adaptive_opts* adaptive, nrrt_accum** out) {
+    if (!adaptive) {
+        if (ctx) ctx->err = "nrrt_accum_create_adaptive: NULL adaptive options";
+        if (out) *out = nullptr;
+        return NRRT_ERR_INVALID;
+    }
+    return accum_create(ctx, cam, opts_in, adaptive, out, "nrrt_accum_create_adaptive");
 }
 
 int nrrt_accum_render(nrrt_accum* a, uint32_t min_samples, nrrt_render_stats* stats) {
@@ -2137,11 +2481,21 @@ int nrrt_accum_render(nrrt_accum* a, uint32_t min_samples, nrrt_render_stats* st
     while (c1 < n_chunks && a->starts[c1] < min_samples) ++c1;  // whole chunks, up to spp
     nrrt_render_stats st;
     std::memset(&st, 0, sizeof st);
-    st.pixels = (uint32_t)(a->n_sums / 3);
-    if (c1 > a->chunks_done) {
+    st.pixels = a->adaptive ? a->n_active : (uint32_t)(a->n_sums / 3);
+    if (c1 > a->chunks_done && (!a->adaptive || a->n_active)) {  // (an adaptive frame with no active pixel is done)
+        AdaptivePass ap;
+        if (a->adaptive)
+            ap = AdaptivePass{a->d_active[a->cur], a->n_active, a->st, a->d_starts, a->test, a->d_keep, a->d_blocks,
+                              a->d_active[a->cur ^ 1], a->d_n_next};
         rc = render_chunks(a->ctx, a->cam, a->opts, a->chunks_done, c1, a->d_sum, 0.0, nullptr, false, false, nullptr,
-                           nullptr, &st, "nrrt_accum_render");
+                           nullptr, &st, "nrrt_accum_render", a->adaptive ? &ap : nullptr);
         if (rc != NRRT_OK) return rc;
+        if (a->adaptive) {  // the only value of the compaction the host needs: 4 bytes per pass
+            nrrt_ctx* ctx = a->ctx;
+            CK(cudaMemcpyAsync(&a->n_active, a->d_n_next, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+            CK(cudaStreamSynchronize(ctx->stream));
+            a->cur ^= 1;
+        }
         a->chunks_done = c1;
     }
     if (stats) *stats = st;
@@ -2149,6 +2503,47 @@ int nrrt_accum_render(nrrt_accum* a, uint32_t min_samples, nrrt_render_stats* st
 }
 
 uint32_t nrrt_accum_samples(const nrrt_accum* a) { return a ? a->starts[a->chunks_done] : 0; }
+
+uint32_t nrrt_accum_active(const nrrt_accum* a) { return a && a->adaptive ? a->n_active : 0; }
+
+// One of an adaptive frame's per-pixel outputs (k_adaptive_map<what>), laid out as nrrt_accum_image lays out the image
+static int adaptive_map(nrrt_accum* a, int what, void* out, uint32_t flags, const char* who) {
+    int rc = accum_check(a, who);
+    if (rc != NRRT_OK) return rc;
+    nrrt_ctx* ctx = a->ctx;
+    if (!a->adaptive || !out) {
+        ctx->err = std::string(who) + (out ? ": not an adaptive frame (nrrt_accum_create_adaptive)" : ": NULL output");
+        return NRRT_ERR_INVALID;
+    }
+    const nrrt_camera& c = a->cam;
+    const nrrt_render_opts& o = a->opts;
+    RenderParams P;  // owned_pixel's fields
+    P.key = make_uint2(0, 0);
+    if (const char* why = work_item_params(P, c.width, c.height, c.samples_per_pixel, o.rank, o.world, o.rows_per_block,
+                                           a->chunks_done, a->chunks_done)) {
+        ctx->err = std::string(who) + ": " + why;
+        return NRRT_ERR_INVALID;
+    }
+    const size_t px_bytes = what == AMAP_SAMPLES ? sizeof(uint32_t) : 3 * sizeof(float);
+    const bool out_dev = (flags & NRRT_RENDER_OUT_DEVICE) != 0, packed = (flags & NRRT_RENDER_OUT_PACKED) != 0;
+    void* d_out = out;
+    if (!out_dev) {
+        if ((rc = ensure_scratch(ctx, std::max<size_t>((size_t)c.width * c.height * px_bytes, 256))) != NRRT_OK) return rc;
+        d_out = ctx->scratch;
+    }
+    if (P.n_owned_pixels) {
+        const unsigned blocks = (P.n_owned_pixels + 255) / 256;
+        if (what == AMAP_IMAGE) k_adaptive_map<AMAP_IMAGE><<<blocks, 256, 0, ctx->stream>>>(c, P, a->st, d_out, packed);
+        else if (what == AMAP_ERROR) k_adaptive_map<AMAP_ERROR><<<blocks, 256, 0, ctx->stream>>>(c, P, a->st, d_out, packed);
+        else k_adaptive_map<AMAP_SAMPLES><<<blocks, 256, 0, ctx->stream>>>(c, P, a->st, d_out, packed);
+        CK(cudaGetLastError());
+    }
+    if (out_dev) {
+        CK(cudaStreamSynchronize(ctx->stream));
+        return NRRT_OK;
+    }
+    return copy_owned_rows(ctx, o, c.width, c.height, packed, d_out, out, px_bytes);
+}
 
 int nrrt_accum_image(nrrt_accum* a, float* out_rgb, uint32_t flags) {
     int rc = accum_check(a, "nrrt_accum_image");
@@ -2158,6 +2553,7 @@ int nrrt_accum_image(nrrt_accum* a, float* out_rgb, uint32_t flags) {
         ctx->err = out_rgb ? "nrrt_accum_image: no samples rendered yet" : "nrrt_accum_image: NULL output";
         return NRRT_ERR_INVALID;
     }
+    if (a->adaptive) return adaptive_map(a, AMAP_IMAGE, out_rgb, flags, "nrrt_accum_image");  // each pixel by its own N
     const nrrt_camera& c = a->cam;
     const nrrt_render_opts& o = a->opts;
     RenderParams P;  // owned_pixel's fields; no chunks: k_resolve divides the sums as they are
@@ -2186,10 +2582,22 @@ int nrrt_accum_image(nrrt_accum* a, float* out_rgb, uint32_t flags) {
     return copy_owned_rows(ctx, o, c.width, c.height, packed, d_fb, out_rgb);
 }
 
+int nrrt_accum_sample_map(nrrt_accum* a, uint32_t* out, uint32_t flags) {
+    return adaptive_map(a, AMAP_SAMPLES, out, flags, "nrrt_accum_sample_map");
+}
+
+int nrrt_accum_error_image(nrrt_accum* a, float* out_rgb, uint32_t flags) {
+    return adaptive_map(a, AMAP_ERROR, out_rgb, flags, "nrrt_accum_error_image");
+}
+
 int nrrt_accum_save(const nrrt_accum* a, double* sums, uint32_t* samples_done) {
     int rc = accum_check(a, "nrrt_accum_save");
     if (rc != NRRT_OK) return rc;
     nrrt_ctx* ctx = a->ctx;
+    if (a->adaptive) {
+        ctx->err = "nrrt_accum_save: an adaptive frame's pixels hold different sample counts (nrrt_accum_adaptive_save)";
+        return NRRT_ERR_INVALID;
+    }
     if ((!sums && a->n_sums) || !samples_done) {
         ctx->err = "nrrt_accum_save: NULL output";
         return NRRT_ERR_INVALID;
@@ -2204,6 +2612,10 @@ int nrrt_accum_restore(nrrt_accum* a, const double* sums, uint32_t samples_done)
     int rc = accum_check(a, "nrrt_accum_restore");
     if (rc != NRRT_OK) return rc;
     nrrt_ctx* ctx = a->ctx;
+    if (a->adaptive) {
+        ctx->err = "nrrt_accum_restore: an adaptive frame is restored with nrrt_accum_adaptive_restore";
+        return NRRT_ERR_INVALID;
+    }
     const auto at = std::find(a->starts.begin(), a->starts.end(), samples_done);
     if (at == a->starts.end()) {
         ctx->err = "nrrt_accum_restore: " + std::to_string(samples_done) + " samples is not a chunk boundary of this frame"
@@ -2220,14 +2632,108 @@ int nrrt_accum_restore(nrrt_accum* a, const double* sums, uint32_t samples_done)
     return NRRT_OK;
 }
 
+int nrrt_adaptive_converged(const double S[3], const double Q[3], uint32_t samples, uint32_t chunks,
+                            const nrrt_adaptive_opts* adaptive) {
+    if (!S || !Q || !adaptive) return 0;
+    return adaptive_converged(S, Q, samples, chunks, *adaptive) ? 1 : 0;
+}
+
+int nrrt_accum_adaptive_save(const nrrt_accum* a, double* sums, double* sumsq, uint32_t* samples) {
+    int rc = accum_check(a, "nrrt_accum_adaptive_save");
+    if (rc != NRRT_OK) return rc;
+    nrrt_ctx* ctx = a->ctx;
+    if (!a->adaptive || (a->n_sums && (!sums || !sumsq || !samples))) {
+        ctx->err = a->adaptive ? "nrrt_accum_adaptive_save: NULL output" : "nrrt_accum_adaptive_save: not an adaptive frame";
+        return NRRT_ERR_INVALID;
+    }
+    if (a->n_sums) {
+        CK(cudaMemcpyAsync(sums, a->st.S, a->n_sums * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaMemcpyAsync(sumsq, a->st.Q, a->n_sums * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaMemcpyAsync(samples, a->st.N, a->n_sums / 3 * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+    }
+    CK(cudaStreamSynchronize(ctx->stream));
+    return NRRT_OK;
+}
+
+int nrrt_accum_adaptive_restore(nrrt_accum* a, const double* sums, const double* sumsq, const uint32_t* samples) {
+    const char* who = "nrrt_accum_adaptive_restore";
+    int rc = accum_check(a, who);
+    if (rc != NRRT_OK) return rc;
+    nrrt_ctx* ctx = a->ctx;
+    const size_t n = a->n_sums / 3;
+    if (!a->adaptive || (n && (!sums || !sumsq || !samples))) {
+        ctx->err = std::string(who) + (a->adaptive ? ": NULL input" : ": not an adaptive frame");
+        return NRRT_ERR_INVALID;
+    }
+    // every N a chunk boundary; the frame's boundary is the largest (0: nothing rendered yet, so every N is 0)
+    const uint32_t n_chunks = (uint32_t)a->starts.size() - 1;
+    std::vector<uint32_t> K(n);
+    uint32_t cb = 0;
+    for (size_t i = 0; i < n; ++i) {
+        const auto at = std::lower_bound(a->starts.begin(), a->starts.end(), samples[i]);
+        if (at == a->starts.end() || *at != samples[i]) {
+            ctx->err = std::string(who) + ": pixel " + std::to_string(i) + " holds " + std::to_string(samples[i]) +
+                       " samples, not a chunk boundary of this frame (nrrt_chunk_starts)";
+            return NRRT_ERR_INVALID;
+        }
+        K[i] = (uint32_t)(at - a->starts.begin());
+        cb = std::max(cb, K[i]);
+        if (K[i] == 0)  // no samples: nothing may be summed yet, or the first pass would add it in
+            for (int ch = 0; ch < 3; ++ch)
+                if (sums[3 * i + ch] != 0.0 || sumsq[3 * i + ch] != 0.0) {
+                    ctx->err = std::string(who) + ": pixel " + std::to_string(i) + " holds no samples but non-zero sums";
+                    return NRRT_ERR_INVALID;
+                }
+    }
+    // pixels below the boundary are retired (they passed the test at their last pass); at the boundary a pixel is
+    // active unless it passed it or has every sample.  Active pixels are listed in owned-pixel order, as a pass does.
+    const nrrt_camera& c = a->cam;
+    const nrrt_render_opts& o = a->opts;
+    RenderParams P;
+    P.key = make_uint2(0, 0);
+    if (const char* why = work_item_params(P, c.width, c.height, c.samples_per_pixel, o.rank, o.world, o.rows_per_block)) {
+        ctx->err = std::string(who) + ": " + why;
+        return NRRT_ERR_INVALID;
+    }
+    std::vector<uint32_t> active;
+    for (uint32_t po = 0; po < P.n_owned_pixels; ++po) {
+        uint32_t x, y, j;
+        owned_pixel(c, P, po, x, y, j);
+        const size_t pix = (size_t)j * c.width + x;
+        const bool conv = adaptive_converged(sums + 3 * pix, sumsq + 3 * pix, samples[pix], K[pix], a->test);
+        if (K[pix] < cb && (K[pix] == 0 || !conv)) {
+            ctx->err = std::string(who) + ": pixel (" + std::to_string(x) + ", " + std::to_string(y) + ") stopped at " +
+                       std::to_string(samples[pix]) + " samples, below the frame's " + std::to_string(a->starts[cb]) +
+                       ", without passing the test";
+            return NRRT_ERR_INVALID;
+        }
+        if (K[pix] == cb && (cb == 0 || (cb < n_chunks && !conv))) active.push_back(po);
+    }
+    if (n) {
+        CK(cudaMemcpyAsync(a->st.S, sums, n * 3 * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+        CK(cudaMemcpyAsync(a->st.Q, sumsq, n * 3 * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+        CK(cudaMemcpyAsync(a->st.N, samples, n * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+        CK(cudaMemcpyAsync(a->st.K, K.data(), n * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+    }
+    if (!active.empty())
+        CK(cudaMemcpyAsync(a->d_active[0], active.data(), active.size() * sizeof(uint32_t), cudaMemcpyHostToDevice,
+                           ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    a->cur = 0;
+    a->n_active = (uint32_t)active.size();
+    a->chunks_done = cb;
+    return NRRT_OK;
+}
+
 void nrrt_accum_free(nrrt_accum* a) {
     if (!a) return;
-    if (a->ctx && a->d_sum) {
+    if (a->ctx) {
         cudaSetDevice(a->ctx->device);
         cudaStreamSynchronize(a->ctx->stream);
-        cudaFree(a->d_sum);
+        accum_release(a);
+    } else {
+        delete a;
     }
-    delete a;
 }
 
 // rows of one rank, packed -> their places in the full image (device-output form of nrrt_render_multi)
@@ -2419,6 +2925,7 @@ size_t nrrt_abi_sizeof(int which) {
         case 16: return sizeof(nrrt_camera_file);
         case 17: return sizeof(nrrt_wnode);
         case 18: return sizeof(nrrt_hit_compact);
+        case 19: return sizeof(nrrt_adaptive_opts);
         default: return 0;
     }
 }

@@ -475,7 +475,7 @@ __device__ __forceinline__ void pool_shade(const DevScene& S, const nrrt_camera&
     wi.x = wi.y = wi.sample_end = 0;
     Sampler smp{RP.key, 0u, 0u};
     if (valid && state != PS_NEED_ITEM) {
-        decode_item(cam, RP, item, wi);
+        decode_item<(F & NRRT_F_ACTIVE) != 0>(cam, RP, item, wi);
         smp.pixel = wi.y * cam.width + wi.x;
         smp.sample = P.cw(PL::CW_SAMPLE, s);
     }
@@ -554,7 +554,7 @@ __device__ __forceinline__ void pool_shade(const DevScene& S, const nrrt_camera&
             P.w(PL::W_CTL, s) = ctl_make(PS_RETIRED, 0, 0, 0);
             return;
         }
-        smp.sample = decode_item(cam, RP, item, wi);
+        smp.sample = decode_item<(F & NRRT_F_ACTIVE) != 0>(cam, RP, item, wi);
         smp.pixel = wi.y * cam.width + wi.x;
         P.st3c(PL::C_SUM, s, mk3(0.0, 0.0, 0.0));
         state = PS_NEED_PATH;

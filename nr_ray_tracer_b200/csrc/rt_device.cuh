@@ -32,6 +32,9 @@
 #define NRRT_F_DIELECTRIC 16u
 #define NRRT_F_MOTION 32u       // moving spheres (SphereBuilder::with_speed): rays carry Ray::time
 #define NRRT_F_ALL 63u
+// Not a scene feature: the launch is an adaptive pass and decodes its work items through RenderParams.active
+// (decode_item<true>).  Plain renders launch instantiations without it.
+#define NRRT_F_ACTIVE 64u
 #ifndef NRRT_STACK_CAP
 #define NRRT_STACK_CAP 32          // traversal stack entries per thread (host validates max_stack)
 #endif

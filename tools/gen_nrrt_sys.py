@@ -19,14 +19,14 @@ STRUCTS = [("nrrt_object", A.Object), ("nrrt_material", A.Material), ("nrrt_text
            ("nrrt_node", A.Node), ("nrrt_box", A.Box), ("nrrt_wnode", A.WNode), ("nrrt_xform", A.Xform),
            ("nrrt_instance", A.Instance), ("nrrt_scene_desc", A.SceneDesc), ("nrrt_hit", A.Hit),
            ("nrrt_hit_compact", A.HitCompact), ("nrrt_trace_stats", A.TraceStats), ("nrrt_render_opts", A.RenderOpts),
-           ("nrrt_render_stats", A.RenderStats), ("nrrt_camera_file", A.CameraFile)]
+           ("nrrt_render_stats", A.RenderStats), ("nrrt_camera_file", A.CameraFile), ("nrrt_adaptive_opts", A.AdaptiveOpts)]
 NAMES = {cls: name for name, cls in STRUCTS}
 SCALARS = {C.c_uint32: "u32", C.c_uint64: "u64", C.c_double: "f64", C.c_float: "f32", C.c_uint8: "u8", C.c_int: "c_int"}
 # which = index accepted by nrrt_abi_sizeof (header order, see include/nrrt.h)
 SIZEOF_ORDER = ["nrrt_object", "nrrt_material", "nrrt_texture", "nrrt_image", "nrrt_graph_desc", "nrrt_camera_config",
                 "nrrt_camera", "nrrt_node", "nrrt_box", "nrrt_xform", "nrrt_instance", "nrrt_scene_desc", "nrrt_hit",
                 "nrrt_trace_stats", "nrrt_render_opts", "nrrt_render_stats", "nrrt_camera_file", "nrrt_wnode",
-                "nrrt_hit_compact"]
+                "nrrt_hit_compact", "nrrt_adaptive_opts"]
 
 
 def rust_type(t, field=""):
@@ -137,6 +137,20 @@ extern "C" {
     pub fn nrrt_accum_save(accum: *const nrrt_accum, sums: *mut f64, samples_done: *mut u32) -> c_int;
     pub fn nrrt_accum_restore(accum: *mut nrrt_accum, sums: *const f64, samples_done: u32) -> c_int;
     pub fn nrrt_accum_free(accum: *mut nrrt_accum);
+    // adaptive sampling: passes render the pixels still active; a pixel retires once its error estimate meets the tolerance
+    pub fn nrrt_accum_create_adaptive(ctx: *mut nrrt_ctx, camera: *const nrrt_camera, opts: *const nrrt_render_opts,
+                                      adaptive: *const nrrt_adaptive_opts, out: *mut *mut nrrt_accum) -> c_int;
+    pub fn nrrt_accum_active(accum: *const nrrt_accum) -> u32;
+    pub fn nrrt_accum_sample_map(accum: *mut nrrt_accum, out: *mut u32, flags: u32) -> c_int;
+    pub fn nrrt_accum_error_image(accum: *mut nrrt_accum, out_rgb: *mut f32, flags: u32) -> c_int;
+    pub fn nrrt_accum_adaptive_save(accum: *const nrrt_accum, sums: *mut f64, sumsq: *mut f64, samples: *mut u32) -> c_int;
+    pub fn nrrt_accum_adaptive_restore(accum: *mut nrrt_accum, sums: *const f64, sumsq: *const f64,
+                                       samples: *const u32) -> c_int;
+    pub fn nrrt_adaptive_converged(s: *const f64, q: *const f64, samples: u32, chunks: u32,
+                                   adaptive: *const nrrt_adaptive_opts) -> c_int;
+    pub fn nrrt_pass_items_active(width: u32, height: u32, samples_per_pixel: u32, rank: u32, world: u32,
+                                  rows_per_block: u32, c0: u32, c1: u32, active: *const u32, n_active: u32, first: u32,
+                                  n: u32, out: *mut u32) -> u32;
     pub fn nrrt_abi_sizeof(which: c_int) -> usize;
 }
 '''

@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Small renders for compute-sanitizer (developer tool, GPU box): every kernel design on a 64x36 Cornell box, the
-pooled and fused kernels on the teapot mesh and the sphere field, scenes whose traversal stacks are full by
-construction (four instance levels, 65536 instances), a fixed-ray batch each.
+pooled and fused kernels on the teapot mesh and the sphere field, an adaptive frame in every design, scenes whose
+traversal stacks are full by construction (four instance levels, 65536 instances), a fixed-ray batch each.
   compute-sanitizer --tool memcheck  python tools/sanitize_run.py
   compute-sanitizer --tool racecheck python tools/sanitize_run.py"""
 import os
@@ -32,6 +32,25 @@ for name, modes in (("cornell-box-scene.json", (A.MODE_FUSED, A.MODE_POOL, A.MOD
     rays = np.concatenate([kat.random_rays(g, 2000), kat.special_rays(g)[:500]])
     hits, _ = ctx.trace_rays(rays)
     print(name, "trace", int((hits["object"] != 0xFFFFFFFF).sum()), flush=True)
+# adaptive frames in every design: the active-list decode, k_resolve_adaptive, the ordered compaction, the per-pixel
+# maps, and a restore
+g = load_scene("scenes/spheres.toml", camera_override=CameraConfig(width=64, height=36, samples_per_pixel=24, ray_max_bounces=50))
+hs = api.HostScene(g)
+ctx.upload(hs)
+cam = api.camera_build(g.camera.to_builder_config())
+ref = None
+for m in (A.MODE_FUSED, A.MODE_POOL, A.MODE_WAVEFRONT, A.MODE_MEGAKERNEL):
+    with ctx.progressive(cam, seed=1, mode=m, adaptive={"rel_error": 0.05, "min_samples": 2}) as p:
+        passes = []
+        while p.active:
+            p.render(p.samples + 1)
+            passes.append(p.active)
+            if len(passes) == 3:
+                p.restore(*p.state())
+        img, err, n = p.image(), p.error_image(), p.sample_map()
+    ref = (img, n) if ref is None else ref
+    assert np.array_equal(img, ref[0]) and np.array_equal(n, ref[1])
+    print("adaptive", A.MODE_NAMES[m], "active per pass", passes, "mean samples", float(n.mean()), flush=True)
 # stacks full by construction (tools/instance_scenes.py): four instance levels at max_stack 32, the LITE pool variant at
 # its per-scene cap (binary stack 24), and 65536 instances (ids past 16 bits in the pooled kernel's chain words)
 for name, g, runs in (("full_stack(32)", S.full_stack(32), ((A.MODE_FUSED, None), (A.MODE_POOL, "0"), (A.MODE_WAVEFRONT, None))),
