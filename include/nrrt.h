@@ -574,10 +574,54 @@ uint32_t nrrt_pass_items_active(uint32_t width, uint32_t height, uint32_t sample
                                 uint32_t world, uint32_t rows_per_block, uint32_t c0, uint32_t c1,
                                 const uint32_t* active, uint32_t n_active, uint32_t first, uint32_t n, uint32_t* out);
 
-/* sizeof() of the ABI structs as compiled (which = 0..19: object, material, texture,
+/* ---- denoising ---------------------------------------------------------------------------------------------------
+ * An extra output of a frame, like nrrt_accum_error_image: the frame's own image, state and kernels are untouched.
+ *
+ * Guides (AOVs).  Per owned pixel, the mean over its samples s = 0 .. n-1 of the first hit of sample s's camera ray (the
+ * render's ray: same Philox counters, so the same jitter, lens point and shutter time), traced on [0.001, inf):
+ *   normal = the hit record's normal (the one shading sees; quirk Q4: a Scale wrapper leaves it in object space),
+ *   albedo = the material texture's colour at the hit (Lambertian, Metal), (1, 1, 1) (Dielectric), the texture colour
+ *            clamped to [0, 1] per channel (DiffuseLight);
+ *   a miss gives normal (0, 0, 0) and albedo = the background clamped to [0, 1].
+ * Summed in f64 in sample order, divided by n, cast to f32: the CPU oracle's restatement (tests/aov_ref.py) bit for bit.
+ *
+ * Filter.  An edge-avoiding a-trous wavelet filter (SVGF form) on the albedo-demodulated image, guided by the normals,
+ * the albedo and the frame's per-pixel error estimate.  Every f32 operation is rounded on its own (no FMA), in this
+ * order.  Per pixel p:  C = (float)(S / N);  e2 = (float)e2 of the adaptive test, +inf where K < 2;  A, Nrm the guides.
+ *   prologue:   a = max(A, 2^-8) per channel;  E = C / a;  v = ((e2_r/(a_r*a_r) + e2_g/(a_g*a_g)) + e2_b/(a_b*a_b)) * (1/9)
+ *   iteration i = 0 .. iterations-1, h = 2^i, from (E, v) of the previous one:
+ *     l = ((E_r + E_g) + E_b) / 3;   sums Sw = SE = Sv = 0;
+ *     taps q = p + h*(dx, dy), dy outer and dx inner over -2..2, taps outside the image skipped;
+ *     k = b[|dx|] * b[|dy|], b = {3/8, 1/4, 1/16};
+ *     centre tap: w = k;  other taps: w = ((k * wn) * wa) * wc with
+ *       wn = max(Nrm_p . Nrm_q, 0) squared 7 times (dot products (x*x' + y*y') + z*z'),
+ *       wa = 1 / (1 + |A_p - A_q|^2 * 64),
+ *       wc = 1 where v_p = +inf, else 1 / (1 + (l_p - l_q)^2 / (sigma_color^2 * v_p + 1e-10)), sigma_color^2 in f32;
+ *       a tap with w * w == 0 adds nothing (w == 0, or w so small that w * w underflows: 0 * inf never reaches
+ *       the sums; the centre's w * w = 81/4096);
+ *     Sw += w;  SE_c += w * E_q,c;  Sv += (w * w) * v_q  (in tap order);   E' = SE / Sw;  v' = Sv / (Sw * Sw)
+ *   epilogue:   out = E' * a per channel.
+ * Sw >= 9/64 (the centre tap), so nothing divides by zero. */
+typedef struct nrrt_denoise_opts {
+    uint32_t iterations;  /* 1..8; 0 -> 5 */
+    uint32_t aov_samples; /* guides over the first n samples, 1..spp; 0 -> min(spp, 16) */
+    float sigma_color;    /* > 0 and finite; 0 -> 4 */
+    uint32_t _pad;
+} nrrt_denoise_opts;
+/* The guides of the frame's first aov_samples samples per pixel (0: min(spp, 16)), f32 RGB each, laid out as
+ * nrrt_accum_image lays out the image (flags NRRT_RENDER_OUT_DEVICE / _PACKED); either output may be NULL.  Works on any
+ * handle, before the first pass too.  The handle computes them on first use for a given aov_samples and keeps them
+ * (24 B per owned pixel, freed with the handle); passes never change them. */
+int nrrt_accum_aov(nrrt_accum* accum, uint32_t aov_samples, float* albedo, float* normal, uint32_t flags);
+/* The filter above on the frame so far, W x H x 3 f32 (NRRT_RENDER_OUT_DEVICE as in nrrt_accum_image; opts may be NULL:
+ * every default).  NRRT_ERR_INVALID for a plain handle (no error estimate), world > 1 or NRRT_RENDER_OUT_PACKED (the
+ * filter reads neighbours across rows), before the first pass, and for options out of range. */
+int nrrt_accum_denoise(nrrt_accum* accum, const nrrt_denoise_opts* opts, float* out_rgb, uint32_t flags);
+
+/* sizeof() of the ABI structs as compiled (which = 0..20: object, material, texture,
  * image, graph_desc, camera_config, camera, node, box, xform, instance, scene_desc, hit, trace_stats,
- * render_opts, render_stats, camera_file, wnode, hit_compact, adaptive_opts) so a binding can verify its mirror of this
- * header. */
+ * render_opts, render_stats, camera_file, wnode, hit_compact, adaptive_opts, denoise_opts) so a binding can verify its
+ * mirror of this header. */
 size_t nrrt_abi_sizeof(int which);
 
 #ifdef __cplusplus

@@ -99,6 +99,8 @@ def lib() -> C.CDLL:
         L.nrrt_pass_items_active.restype = C.c_uint32
         L.nrrt_pass_items_active.argtypes = [C.c_uint32] * 8 + [C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32,
                                                                  C.POINTER(C.c_uint32)]
+        L.nrrt_accum_aov.argtypes = [C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint32]
+        L.nrrt_accum_denoise.argtypes = [C.c_void_p, C.POINTER(A.DenoiseOpts), C.c_void_p, C.c_uint32]
         L.nrrt_abi_sizeof.restype = C.c_size_t
         L.nrrt_abi_sizeof.argtypes = [C.c_int]
         _lib = L
@@ -107,7 +109,7 @@ def lib() -> C.CDLL:
 
 ABI_STRUCTS = [A.Object, A.Material, A.Texture, A.Image, A.GraphDesc, A.CameraConfig, A.Camera, A.Node, A.Box,
                A.Xform, A.Instance, A.SceneDesc, A.Hit, A.TraceStats, A.RenderOpts, A.RenderStats, A.CameraFile, A.WNode,
-               A.HitCompact, A.AdaptiveOpts]
+               A.HitCompact, A.AdaptiveOpts, A.DenoiseOpts]
 
 
 def chunk_starts(samples_per_pixel: int, total_pixels: int):
@@ -505,6 +507,46 @@ class Progressive:
         pixel holds fewer than two chunks."""
         return self._map(lib().nrrt_accum_error_image, (3,), np.float32, packed, out_device_ptr)
 
+    def aov(self, samples: Optional[int] = None, packed: bool = False, out_device_ptr: Optional[int] = None):
+        """Denoising guides: the mean first-hit albedo and normal of each pixel's first `samples` samples (None:
+        min(spp, 16)), (albedo, normal) as (H, W, 3) f32 laid out as image().  out_device_ptr: two device buffers
+        (albedo, normal) of that size; returns None then.  Computed once per sample count and kept by the frame."""
+        n = 0 if samples is None else int(samples)
+        if samples is not None and n < 1:
+            raise ValueError("samples must be >= 1")
+        flags = (A.RENDER_OUT_DEVICE if out_device_ptr is not None else 0) | (A.RENDER_OUT_PACKED if packed else 0)
+        if out_device_ptr is not None:
+            pa, pn = out_device_ptr
+            self.ctx._check(lib().nrrt_accum_aov(self._h, n, C.c_void_p(pa), C.c_void_p(pn), flags))
+            return None
+        shape = ((self.rows if packed else self.camera.height), self.camera.width, 3)
+        albedo, normal = np.zeros(shape, np.float32), np.zeros(shape, np.float32)
+        self.ctx._check(lib().nrrt_accum_aov(self._h, n, C.c_void_p(albedo.ctypes.data), C.c_void_p(normal.ctypes.data),
+                                             flags))
+        return albedo, normal
+
+    def denoised(self, iterations: int = 5, sigma_color: float = 4.0, aov_samples: Optional[int] = None,
+                 out: Optional[np.ndarray] = None, out_device_ptr: Optional[int] = None) -> Optional[np.ndarray]:
+        """The frame so far through the a-trous filter (nrrt_accum_denoise): (H, W, 3) f32, or None for device output.
+        Needs an adaptive frame (its per-pixel error estimate guides the filter) on one GPU (world == 1)."""
+        if not 1 <= int(iterations) <= 8:
+            raise ValueError("iterations must be 1..8")
+        if not (np.isfinite(sigma_color) and sigma_color > 0):
+            raise ValueError("sigma_color must be finite and > 0")
+        if aov_samples is not None and int(aov_samples) < 1:
+            raise ValueError("aov_samples must be >= 1")
+        opts = A.DenoiseOpts(iterations=int(iterations), aov_samples=0 if aov_samples is None else int(aov_samples),
+                             sigma_color=float(sigma_color))
+        if out_device_ptr is not None:
+            self.ctx._check(lib().nrrt_accum_denoise(self._h, C.byref(opts), C.c_void_p(out_device_ptr),
+                                                     A.RENDER_OUT_DEVICE))
+            return None
+        if out is None:
+            out = np.zeros((self.camera.height, self.camera.width, 3), dtype=np.float32)
+        assert out.dtype == np.float32 and out.flags.c_contiguous and out.size == self.camera.height * self.camera.width * 3
+        self.ctx._check(lib().nrrt_accum_denoise(self._h, C.byref(opts), C.c_void_p(out.ctypes.data), 0))
+        return out
+
     def state(self):
         """What restore() takes: (samples done, f64 sums (owned rows, W, 3) in owned-row order), or for an adaptive
         frame (sums, sums of squares (owned rows, W, 3) f64, samples (owned rows, W) uint32)."""
@@ -611,15 +653,35 @@ class Scene:
             raise ValueError("every must be >= 1")
         ad = {"rel_error": rel_error, "abs_error": abs_error, "min_samples": min_samples}
         with self.ctx.progressive(self.camera, adaptive=ad, **kw) as p:
-            spp = p.samples_per_pixel
-            starts = chunk_starts(spp, self.camera.width * self.camera.height)
-            k = next((i for i, s in enumerate(starts) if i and s >= p.adaptive.min_samples), len(starts) - 1)
-            while p.active:
-                done = p.samples
-                if every is None:
-                    target = starts[min(k, len(starts) - 1)]
-                    k *= 2
-                else:
-                    target = (done // every + 1) * every
-                self.last_stats = p.render(min(target, spp))
+            for _ in self._adaptive_passes(p, every):
                 yield p.samples, p.active, p.image()
+
+    def _adaptive_passes(self, p: Progressive, every: Optional[int]):
+        """Runs render_adaptive's passes on the adaptive frame p, yielding after each one."""
+        spp = p.samples_per_pixel
+        starts = chunk_starts(spp, self.camera.width * self.camera.height)
+        k = next((i for i, s in enumerate(starts) if i and s >= p.adaptive.min_samples), len(starts) - 1)
+        while p.active:
+            done = p.samples
+            if every is None:
+                target = starts[min(k, len(starts) - 1)]
+                k *= 2
+            else:
+                target = (done // every + 1) * every
+            self.last_stats = p.render(min(target, spp))
+            yield
+
+    def render_denoised(self, rel_error: float = 0.0, abs_error: float = 0.0, iterations: int = 5,
+                        sigma_color: float = 4.0, aov_samples: Optional[int] = None, **kw):
+        """Scene::render followed by the a-trous filter (Progressive.denoised): returns (image, denoised), both (H, W, 3)
+        f32.  The frame is adaptive with the given tolerances and render_adaptive's passes; with both tolerances 0 it is
+        one pass and `image` is render()'s image bit for bit.  kw: Context.progressive's options (seed, mode, ...) and
+        min_samples."""
+        ad = {"rel_error": rel_error, "abs_error": abs_error, "min_samples": kw.pop("min_samples", None)}
+        with self.ctx.progressive(self.camera, adaptive=ad, **kw) as p:
+            if rel_error == 0.0 and abs_error == 0.0:
+                self.last_stats = p.render(p.samples_per_pixel)
+            else:
+                for _ in self._adaptive_passes(p, None):
+                    pass
+            return p.image(), p.denoised(iterations=iterations, sigma_color=sigma_color, aov_samples=aov_samples)

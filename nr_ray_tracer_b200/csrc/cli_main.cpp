@@ -6,7 +6,7 @@
 // Flags and NR_RT_CAMERA_* environment fallbacks follow ray-tracer/src/cli.rs:113-270 (field of view and defocus
 // angle in degrees; image size needs exactly two of width / height / aspect ratio; default output out.png,
 // default gamma 0.5).  Additions: --seed, --mode auto|pool|fused|wavefront|megakernel, --device N, --gpus N,
-// --preview-every N, --adaptive-error REL [--adaptive-abs-error ABS] [--adaptive-min-samples N].
+// --preview-every N, --adaptive-error REL [--adaptive-abs-error ABS] [--adaptive-min-samples N], --denoise.
 // Encoders available without external libraries: .png (stored/uncompressed deflate) and .ppm.
 #include <algorithm>
 #include <cerrno>
@@ -181,6 +181,10 @@ static void usage() {
         "      --adaptive-min-samples <N> test a pixel only from N samples on (default: the first work-chunk boundary at\n"
         "                                 or above 1/8 of the samples per pixel).  Passes end at doubling chunk counts\n"
         "                                 from there, or as --preview-every sets them\n"
+        "      --denoise                  write the image through the edge-avoiding a-trous filter, guided by first-hit\n"
+        "                                 albedo and normals and each pixel's error estimate (an adaptive frame, with\n"
+        "                                 tolerance 0 unless --adaptive-error is given; previews are denoised too; one\n"
+        "                                 GPU only)\n"
         "  -v, --verbose                  print timing\n"
         "Every camera option falls back to NR_RT_CAMERA_<NAME> (e.g. NR_RT_CAMERA_SAMPLES_PER_PIXEL).");
 }
@@ -225,7 +229,7 @@ int main(int argc, char** argv) {
     bool force = false, verbose = false;
     float gamma = 0.5f;  // constants.rs:1
     uint64_t seed = 0, preview_every = 0, adaptive_min = 0;
-    bool adaptive = false, adaptive_min_set = false, adaptive_abs_set = false;
+    bool adaptive = false, adaptive_min_set = false, adaptive_abs_set = false, denoise = false;
     nrrt_adaptive_opts ad;
     std::memset(&ad, 0, sizeof ad);
     int device = 0, gpus = 1;
@@ -298,6 +302,7 @@ int main(int argc, char** argv) {
             return 0;
         }
         if (a == "-f" || a == "--force-overwrite") force = true;
+        else if (a == "--denoise") denoise = true;
         else if (a == "-v" || a == "--verbose") verbose = true;
         else if (a == "-o" || a == "--output") output = need();
         else if (a == "--gamma-value") {
@@ -357,6 +362,8 @@ int main(int argc, char** argv) {
         die(std::string(adaptive_abs_set ? "--adaptive-abs-error" : "--adaptive-min-samples") + " needs --adaptive-error");
     if (adaptive && gpus > 1)
         die("--adaptive-error renders on one GPU: it cannot be combined with --gpus " + std::to_string(gpus));
+    if (denoise && gpus > 1)
+        die("--denoise renders on one GPU: it cannot be combined with --gpus " + std::to_string(gpus));
     auto ends = [&](const char* suf) {
         size_t n = std::strlen(suf);
         return output.size() >= n && output.compare(output.size() - n, n, suf) == 0;
@@ -411,11 +418,13 @@ int main(int argc, char** argv) {
         if (nrrt_render_multi(devs.data(), gpus, nrrt_host_scene_desc(hs), &cam, &opts, image.data(),
                               verbose ? on_progress : nullptr, nullptr, &st, msg, sizeof msg) != NRRT_OK)
             die(msg);
-    } else if (preview_every || adaptive) {
+    } else if (preview_every || adaptive || denoise) {
         // progressive: each pass renders up to the next multiple of N samples (rounded up to a chunk boundary), then the
         // image so far replaces the output file; the last pass completes the frame, which is nrrt_render's bit for bit.
         // Adaptive: the passes render the pixels still active only, and end at doubling chunk counts unless
-        // --preview-every sets them; the frame is finished when no pixel is active.
+        // --preview-every sets them; the frame is finished when no pixel is active.  --denoise: an adaptive frame (tolerance
+        // 0 unless --adaptive-error is given, and then one pass unless --preview-every sets them) whose images go
+        // through nrrt_accum_denoise.
         std::fclose(out);  // (opened above only for the create-new check: every image goes through replace_image)
         out = nullptr;
         nrrt_accum* acc = nullptr;
@@ -423,7 +432,7 @@ int main(int argc, char** argv) {
         std::vector<uint32_t> starts(65);
         const uint32_t n_chunks = nrrt_chunk_starts(spp, (uint64_t)cam.width * cam.height, starts.data(), 65);
         uint32_t k = 1;  // chunk count the next adaptive pass ends on (without --preview-every)
-        if (adaptive) {
+        if (adaptive || denoise) {
             while (k < n_chunks && 8ull * starts[k] < spp) ++k;  // default: the first boundary at or above spp / 8
             ad.min_samples = adaptive_min_set ? (uint32_t)adaptive_min : starts[k];
             k = 1;
@@ -432,7 +441,11 @@ int main(int argc, char** argv) {
         } else if (nrrt_accum_create(ctx, &cam, &opts, &acc) != NRRT_OK) {
             die(nrrt_last_error(ctx));
         }
-        auto more = [&] { return adaptive ? nrrt_accum_active(acc) > 0 : nrrt_accum_samples(acc) < spp; };
+        if (denoise && !adaptive) k = n_chunks;  // tolerance 0: no pixel retires, so one pass renders the frame
+        auto more = [&] { return adaptive || denoise ? nrrt_accum_active(acc) > 0 : nrrt_accum_samples(acc) < spp; };
+        auto frame_image = [&] {
+            return denoise ? nrrt_accum_denoise(acc, nullptr, image.data(), 0) : nrrt_accum_image(acc, image.data(), 0);
+        };
         std::vector<uint8_t> preview(image.size());
         std::memset(&st, 0, sizeof st);
         while (more()) {
@@ -454,13 +467,13 @@ int main(int argc, char** argv) {
             else if (verbose)
                 std::fprintf(stderr, "pass: %u / %u samples  (%.3f s)\n", done, spp, secs);
             if (preview_every && more()) {
-                if (nrrt_accum_image(acc, image.data(), 0) != NRRT_OK ||
+                if (frame_image() != NRRT_OK ||
                     nrrt_encode_rgb8(ctx, image.data(), cam.width, cam.height, gamma, 0, preview.data()) != NRRT_OK)
                     die(nrrt_last_error(ctx));
                 replace_image(output, png, preview.data(), cam.width, cam.height);
             }
         }
-        if (nrrt_accum_image(acc, image.data(), 0) != NRRT_OK) die(nrrt_last_error(ctx));
+        if (frame_image() != NRRT_OK) die(nrrt_last_error(ctx));
         nrrt_accum_free(acc);
     } else if (nrrt_render(ctx, &cam, &opts, image.data(), verbose ? on_progress : nullptr, nullptr, &st) != NRRT_OK)
         die(nrrt_last_error(ctx));

@@ -529,6 +529,150 @@ __global__ void k_adaptive_map(const __grid_constant__ nrrt_camera cam, const __
     }
 }
 
+// ---- denoising (include/nrrt.h): first-hit guides and the a-trous filter
+// The albedo guide of a hit: the colour the material multiplies a path by, (1, 1, 1) for a dielectric, and for a
+// light its texture colour clamped to [0, 1] (its emission is unbounded; a guide compares colours).
+__device__ __forceinline__ d3 clamp01_3(d3 c) {
+    return mk3(fmin(fmax(c.x, 0.0), 1.0), fmin(fmax(c.y, 0.0), 1.0), fmin(fmax(c.z, 0.0), 1.0));
+}
+__device__ __forceinline__ d3 material_albedo(const DevScene& S, const HitRec& h) {
+    NRRT_CHECK(h.material < S.n_materials, "material index");
+    const nrrt_material* m = &S.materials[h.material];
+    if (m->kind == NRRT_MAT_DIELECTRIC) return mk3(1.0, 1.0, 1.0);
+    const d3 c = texture_color(S, m->texture, h.u, h.v, h.point);
+    return m->kind == NRRT_MAT_DIFFUSE_LIGHT ? clamp01_3(c) : c;
+}
+
+// One thread per owned pixel: albedo and normal of the first hit of the pixel's samples [0, n), each sample's camera ray
+// being the render's (same Philox counters, so the same jitter, lens point and shutter time), summed in f64 in sample
+// order and divided by n.  A miss gives the background clamped to [0, 1] and a zero normal.  Owned rows packed.
+__global__ void __launch_bounds__(NRRT_BLOCK)
+k_aov(const __grid_constant__ DevScene S, const __grid_constant__ nrrt_camera cam, const __grid_constant__ RenderParams P,
+      uint32_t n, float* __restrict__ albedo, float* __restrict__ normal) {
+    extern __shared__ uint32_t s_stack[];
+    const uint32_t po = blockIdx.x * blockDim.x + threadIdx.x;
+    const bool valid = po < P.n_owned_pixels;  // no early return: trace_closest votes across the whole warp
+    uint32_t x = 0, y = 0, j = 0;
+    if (valid) owned_pixel(cam, P, po, x, y, j);
+    Sampler smp{P.key, y * cam.width + x, 0u};
+    d3 sa = mk3(0.0, 0.0, 0.0), sn = sa;
+    TraceCounters tc{0, 0, 0, 0, 0};
+    for (uint32_t s = 0; s < n; ++s) {
+        smp.sample = s;
+        d3 o = mk3(0.0, 0.0, 0.0), d = o;
+        double time = 0.0;
+        if (valid) camera_ray<true>(cam, x, y, smp, o, d, time);
+        HitId h;
+        trace_closest<false, false>(S, o, d, time, 0.001, NRRT_INF, s_stack + threadIdx.x, NRRT_BLOCK, h, &tc, valid);
+        if (!valid) continue;
+        if (h.prim == NRRT_REF_NONE) {
+            sa = add3(sa, clamp01_3(ld3(cam.background)));
+            sn = add3(sn, mk3(0.0, 0.0, 0.0));
+        } else {
+            HitRec rec;
+            resolve_hit(S, h, o, d, time, true, rec);
+            sa = add3(sa, material_albedo(S, rec));
+            sn = add3(sn, rec.normal);
+        }
+    }
+    if (!valid) return;
+    const size_t b = ((size_t)j * cam.width + x) * 3;
+    NRRT_CHECK(b + 2 < (size_t)P.n_owned_pixels * 3, "guide index");
+    const d3 ma = div3(sa, (double)n), mn = div3(sn, (double)n);
+    albedo[b] = (float)ma.x, albedo[b + 1] = (float)ma.y, albedo[b + 2] = (float)ma.z;
+    normal[b] = (float)mn.x, normal[b + 1] = (float)mn.y, normal[b + 2] = (float)mn.z;
+}
+
+// The filter on a whole W x H image (one device, rows in image order).  Every f32 operation is an _rn intrinsic, so no
+// FMA contraction changes a rounding and a float32 numpy restatement (tests/denoise_ref.py) gives the same bits.
+#define NRRT_DENOISE_MIN_ALBEDO 0.00390625f  // 2^-8: albedo floor of the demodulation
+#define NRRT_DENOISE_EPS 1e-10f              // keeps the colour weight's denominator positive where v = 0
+// Prologue: E = C / a per channel and the variance of its luminance, v, from the adaptive state (ev[i] = E, v).
+// C = S / N as k_adaptive_map<AMAP_IMAGE> writes it; v = +inf where K < 2 (no error estimate).
+__global__ void k_denoise_init(uint32_t n_pixels, AdaptiveState A, const float* __restrict__ albedo,
+                               float4* __restrict__ ev) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_pixels) return;
+    const uint32_t N = A.N[i], K = A.K[i];
+    float E[3], v = 0.0f;
+    for (int ch = 0; ch < 3; ++ch) {
+        const float C = (float)__ddiv_rn(A.S[3 * i + ch], (double)N);
+        const float e2 = K < 2 ? __int_as_float(0x7f800000) : (float)adaptive_e2(A.S[3 * i + ch], A.Q[3 * i + ch], N, K);
+        const float a = fmaxf(albedo[3 * i + ch], NRRT_DENOISE_MIN_ALBEDO);
+        E[ch] = __fdiv_rn(C, a);
+        const float t = __fdiv_rn(e2, __fmul_rn(a, a));
+        v = ch == 0 ? t : __fadd_rn(v, t);
+    }
+    ev[i] = make_float4(E[0], E[1], E[2], __fmul_rn(v, 1.0f / 9.0f));
+}
+__device__ __forceinline__ float denoise_luma(float4 e) { return __fdiv_rn(__fadd_rn(__fadd_rn(e.x, e.y), e.z), 3.0f); }
+__device__ __forceinline__ float dot3f(float ax, float ay, float az, float bx, float by, float bz) {
+    return __fadd_rn(__fadd_rn(__fmul_rn(ax, bx), __fmul_rn(ay, by)), __fmul_rn(az, bz));
+}
+// Iteration with tap spacing h: 5 x 5 taps q = p + h (dx, dy), dy outer, dx inner, taps outside the image skipped.
+// LAST: also the epilogue, out = E' * max(A, 2^-8) as RGB f32.
+template <bool LAST>
+__global__ void k_denoise_step(uint32_t W, uint32_t H, uint32_t h, float sigma2, const float4* __restrict__ in,
+                               float4* __restrict__ out_ev, const float* __restrict__ albedo,
+                               const float* __restrict__ normal, float* __restrict__ out_rgb) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= W * H) return;
+    const int y = (int)(i / W), x = (int)(i - (uint32_t)y * W), hh = (int)h;
+    const float4 p = in[i];
+    const float lp = denoise_luma(p);
+    const float apr = albedo[3 * i], apg = albedo[3 * i + 1], apb = albedo[3 * i + 2];
+    const float npx = normal[3 * i], npy = normal[3 * i + 1], npz = normal[3 * i + 2];
+    const bool no_estimate = p.w == __int_as_float(0x7f800000);
+    const float den = __fadd_rn(__fmul_rn(sigma2, p.w), NRRT_DENOISE_EPS);
+    const float bk[3] = {0.375f, 0.25f, 0.0625f};
+    float sw = 0.0f, sr = 0.0f, sg = 0.0f, sb = 0.0f, sv = 0.0f;
+#pragma unroll
+    for (int dy = -2; dy <= 2; ++dy) {
+        const int qy = y + dy * hh;
+        if (qy < 0 || qy >= (int)H) continue;
+#pragma unroll
+        for (int dx = -2; dx <= 2; ++dx) {
+            const int qx = x + dx * hh;
+            if (qx < 0 || qx >= (int)W) continue;
+            const uint32_t q = (uint32_t)qy * W + (uint32_t)qx;
+            NRRT_CHECK(q < W * H, "denoise tap index");
+            const float k = __fmul_rn(bk[dx < 0 ? -dx : dx], bk[dy < 0 ? -dy : dy]);
+            const float4 e = in[q];
+            float w = k, ww;
+            if (dx != 0 || dy != 0) {
+                float wn = fmaxf(dot3f(npx, npy, npz, normal[3 * q], normal[3 * q + 1], normal[3 * q + 2]), 0.0f);
+#pragma unroll
+                for (int r = 0; r < 7; ++r) wn = __fmul_rn(wn, wn);  // ^128
+                const float dr = __fsub_rn(apr, albedo[3 * q]), dg = __fsub_rn(apg, albedo[3 * q + 1]),
+                            db = __fsub_rn(apb, albedo[3 * q + 2]);
+                const float wa = __fdiv_rn(1.0f, __fadd_rn(1.0f, __fmul_rn(dot3f(dr, dg, db, dr, dg, db), 64.0f)));
+                float wc = 1.0f;
+                if (!no_estimate) {
+                    const float dl = __fsub_rn(lp, denoise_luma(e));
+                    wc = __fdiv_rn(1.0f, __fadd_rn(1.0f, __fdiv_rn(__fmul_rn(dl, dl), den)));
+                }
+                w = __fmul_rn(__fmul_rn(__fmul_rn(k, wn), wa), wc);
+            }
+            ww = __fmul_rn(w, w);
+            if (ww == 0.0f) continue;  // a rule, not a shortcut: w * w may underflow, and 0 * inf must not reach the sums
+
+            sw = __fadd_rn(sw, w);
+            sr = __fadd_rn(sr, __fmul_rn(w, e.x));
+            sg = __fadd_rn(sg, __fmul_rn(w, e.y));
+            sb = __fadd_rn(sb, __fmul_rn(w, e.z));
+            sv = __fadd_rn(sv, __fmul_rn(ww, e.w));
+        }
+    }
+    const float er = __fdiv_rn(sr, sw), eg = __fdiv_rn(sg, sw), eb = __fdiv_rn(sb, sw);
+    if (LAST) {
+        out_rgb[3 * i] = __fmul_rn(er, fmaxf(apr, NRRT_DENOISE_MIN_ALBEDO));
+        out_rgb[3 * i + 1] = __fmul_rn(eg, fmaxf(apg, NRRT_DENOISE_MIN_ALBEDO));
+        out_rgb[3 * i + 2] = __fmul_rn(eb, fmaxf(apb, NRRT_DENOISE_MIN_ALBEDO));
+    } else {
+        out_ev[i] = make_float4(er, eg, eb, __fdiv_rn(sv, __fmul_rn(sw, sw)));
+    }
+}
+
 __global__ void k_iota(uint32_t* __restrict__ out, uint32_t n) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) out[i] = i;
@@ -2352,6 +2496,9 @@ struct nrrt_accum {
     uint32_t* d_blocks = nullptr;   // compaction block counts
     uint32_t* d_n_next = nullptr;   // compaction result count
     uint32_t* d_starts = nullptr;   // starts on the device
+    // guides (nrrt_accum_aov), computed on first use: albedo then normal, 3 f32 each per owned pixel, owned rows packed
+    float* d_aov = nullptr;
+    uint32_t aov_n = 0;             // the samples per pixel they average (0: not computed)
 };
 
 // the accumulator's context is usable and still holds the scene the accumulator was created for
@@ -2369,6 +2516,7 @@ static int accum_check(const nrrt_accum* a, const char* who) {
 static void accum_release(nrrt_accum* a) {
     if (a->d_sum) cudaFree(a->d_sum);
     if (a->d_ad) cudaFree(a->d_ad);
+    if (a->d_aov) cudaFree(a->d_aov);
     delete a;
 }
 
@@ -2903,6 +3051,135 @@ int nrrt_encode_rgb8(nrrt_ctx* ctx, const float* rgb, uint32_t width, uint32_t h
     return NRRT_OK;
 }
 
+// ---- denoising: guides of a frame and the filter on it
+// aov_samples as given (0: min(spp, 16)), or 0 when it is out of range
+static uint32_t aov_samples_of(const nrrt_accum* a, uint32_t aov_samples) {
+    const uint32_t spp = a->cam.samples_per_pixel;
+    if (aov_samples == 0) return std::min<uint32_t>(spp, 16);
+    return aov_samples <= spp ? aov_samples : 0;
+}
+
+// The frame's guides over its first n samples per pixel in a->d_aov (computed unless they are there already)
+static int accum_guides(nrrt_accum* a, uint32_t n, const char* who) {
+    nrrt_ctx* ctx = a->ctx;
+    if (a->aov_n == n) return NRRT_OK;
+    const nrrt_camera& c = a->cam;
+    const nrrt_render_opts& o = a->opts;
+    RenderParams P;
+    P.key = make_uint2((uint32_t)o.seed, (uint32_t)(o.seed >> 32));
+    if (const char* why = work_item_params(P, c.width, c.height, c.samples_per_pixel, o.rank, o.world, o.rows_per_block)) {
+        ctx->err = std::string(who) + ": " + why;
+        return NRRT_ERR_INVALID;
+    }
+    const size_t n_px = a->n_sums / 3;
+    if (!a->d_aov) CK(cudaMalloc((void**)&a->d_aov, std::max<size_t>(n_px * 6 * sizeof(float), 256)));
+    if (n_px) {
+        const size_t smem = (size_t)NRRT_BLOCK * NRRT_STACK_CAP * sizeof(uint32_t);
+        k_aov<<<(unsigned)((n_px + NRRT_BLOCK - 1) / NRRT_BLOCK), NRRT_BLOCK, smem, ctx->stream>>>(
+            ctx->dev, c, P, n, a->d_aov, a->d_aov + n_px * 3);
+        CK(cudaGetLastError());
+    }
+    CK(cudaStreamSynchronize(ctx->stream));
+    a->aov_n = n;
+    return NRRT_OK;
+}
+
+// An RGB f32 buffer in owned-row order (device) to the caller's buffer laid out as nrrt_accum_image lays out the image
+static int place_owned_rgb(nrrt_ctx* ctx, const nrrt_accum* a, const float* d_packed, float* out, uint32_t flags) {
+    const nrrt_render_opts& o = a->opts;
+    const uint32_t W = a->cam.width, rows = owned_rows(a->cam.height, o.rank, o.world, o.rows_per_block);
+    const bool out_dev = (flags & NRRT_RENDER_OUT_DEVICE) != 0, packed = (flags & NRRT_RENDER_OUT_PACKED) != 0;
+    const size_t row_floats = (size_t)W * 3;
+    if (packed || o.world == 1) {  // the owned rows are the image rows (or the packed layout is asked for)
+        if (rows)
+            CK(cudaMemcpyAsync(out, d_packed, rows * row_floats * sizeof(float),
+                               out_dev ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, ctx->stream));
+    } else if (out_dev) {
+        if (rows) {
+            const size_t n = rows * row_floats;
+            k_place_rows<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(d_packed, out, (uint32_t)row_floats, rows,
+                                                                               o.rank, o.world, o.rows_per_block);
+            CK(cudaGetLastError());
+        }
+    } else {
+        std::vector<float> host(rows * row_floats);
+        if (rows) CK(cudaMemcpyAsync(host.data(), d_packed, host.size() * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+        for (uint32_t k = 0; k < rows; ++k) {  // packed row k = row k % R of the rank's k / R-th block
+            const uint32_t R = o.rows_per_block, y = (k / R * o.world + o.rank) * R + k % R;
+            std::memcpy(out + (size_t)y * row_floats, host.data() + (size_t)k * row_floats, row_floats * sizeof(float));
+        }
+    }
+    CK(cudaStreamSynchronize(ctx->stream));
+    return NRRT_OK;
+}
+
+int nrrt_accum_aov(nrrt_accum* a, uint32_t aov_samples, float* albedo, float* normal, uint32_t flags) {
+    const char* who = "nrrt_accum_aov";
+    int rc = accum_check(a, who);
+    if (rc != NRRT_OK) return rc;
+    nrrt_ctx* ctx = a->ctx;
+    const uint32_t n = aov_samples_of(a, aov_samples);
+    if (n == 0) {
+        ctx->err = std::string(who) + ": aov_samples must be at most the frame's samples per pixel";
+        return NRRT_ERR_INVALID;
+    }
+    if ((rc = accum_guides(a, n, who)) != NRRT_OK) return rc;
+    const size_t n_px = a->n_sums / 3;
+    if (albedo && (rc = place_owned_rgb(ctx, a, a->d_aov, albedo, flags)) != NRRT_OK) return rc;
+    if (normal && (rc = place_owned_rgb(ctx, a, a->d_aov + n_px * 3, normal, flags)) != NRRT_OK) return rc;
+    return NRRT_OK;
+}
+
+int nrrt_accum_denoise(nrrt_accum* a, const nrrt_denoise_opts* opts, float* out_rgb, uint32_t flags) {
+    const char* who = "nrrt_accum_denoise";
+    int rc = accum_check(a, who);
+    if (rc != NRRT_OK) return rc;
+    nrrt_ctx* ctx = a->ctx;
+    nrrt_denoise_opts d;
+    std::memset(&d, 0, sizeof d);
+    if (opts) d = *opts;
+    const uint32_t iterations = d.iterations ? d.iterations : 5, n = aov_samples_of(a, d.aov_samples);
+    const float sigma = d.sigma_color == 0.0f ? 4.0f : d.sigma_color;
+    const char* why = nullptr;
+    if (!a->adaptive) why = "needs an adaptive frame (nrrt_accum_create_adaptive): the filter reads its error estimate";
+    else if (a->opts.world > 1) why = "the filter needs the whole image on one context (world == 1)";
+    else if (flags & NRRT_RENDER_OUT_PACKED) why = "the filter writes the whole image (NRRT_RENDER_OUT_PACKED is refused)";
+    else if (!out_rgb) why = "NULL output";
+    else if (a->chunks_done == 0) why = "no samples rendered yet";
+    else if (iterations > 8) why = "iterations must be 1..8";
+    else if (n == 0) why = "aov_samples must be at most the frame's samples per pixel";
+    else if (!(std::isfinite(sigma) && sigma > 0.0f)) why = "sigma_color must be finite and > 0";
+    if (why) {
+        ctx->err = std::string(who) + ": " + why;
+        return NRRT_ERR_INVALID;
+    }
+    if ((rc = accum_guides(a, n, who)) != NRRT_OK) return rc;
+    const uint32_t W = a->cam.width, H = a->cam.height, n_px = W * H;
+    const bool out_dev = (flags & NRRT_RENDER_OUT_DEVICE) != 0;
+    const size_t ev_bytes = ((size_t)n_px * sizeof(float4) + 255) & ~(size_t)255;
+    if ((rc = ensure_scratch(ctx, 2 * ev_bytes + (out_dev ? 0 : (size_t)n_px * 3 * sizeof(float)))) != NRRT_OK) return rc;
+    float4* ev[2] = {(float4*)ctx->scratch, (float4*)((char*)ctx->scratch + ev_bytes)};
+    float* d_out = out_dev ? out_rgb : (float*)((char*)ctx->scratch + 2 * ev_bytes);
+    const float* albedo = a->d_aov;
+    const float* normal = a->d_aov + (size_t)n_px * 3;
+    const unsigned blocks = (n_px + 255) / 256;
+    k_denoise_init<<<blocks, 256, 0, ctx->stream>>>(n_px, a->st, albedo, ev[0]);
+    CK(cudaGetLastError());
+    for (uint32_t it = 0; it < iterations; ++it) {
+        const float4* in = ev[it & 1];
+        float4* nxt = ev[(it & 1) ^ 1];
+        if (it + 1 < iterations)
+            k_denoise_step<false><<<blocks, 256, 0, ctx->stream>>>(W, H, 1u << it, sigma * sigma, in, nxt, albedo, normal, nullptr);
+        else
+            k_denoise_step<true><<<blocks, 256, 0, ctx->stream>>>(W, H, 1u << it, sigma * sigma, in, nullptr, albedo, normal, d_out);
+        CK(cudaGetLastError());
+    }
+    if (!out_dev) CK(cudaMemcpyAsync(out_rgb, d_out, (size_t)n_px * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return NRRT_OK;
+}
+
 // struct sizes, so bindings can verify their mirror of the header
 size_t nrrt_abi_sizeof(int which) {
     switch (which) {
@@ -2926,6 +3203,7 @@ size_t nrrt_abi_sizeof(int which) {
         case 17: return sizeof(nrrt_wnode);
         case 18: return sizeof(nrrt_hit_compact);
         case 19: return sizeof(nrrt_adaptive_opts);
+        case 20: return sizeof(nrrt_denoise_opts);
         default: return 0;
     }
 }

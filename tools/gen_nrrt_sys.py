@@ -19,14 +19,15 @@ STRUCTS = [("nrrt_object", A.Object), ("nrrt_material", A.Material), ("nrrt_text
            ("nrrt_node", A.Node), ("nrrt_box", A.Box), ("nrrt_wnode", A.WNode), ("nrrt_xform", A.Xform),
            ("nrrt_instance", A.Instance), ("nrrt_scene_desc", A.SceneDesc), ("nrrt_hit", A.Hit),
            ("nrrt_hit_compact", A.HitCompact), ("nrrt_trace_stats", A.TraceStats), ("nrrt_render_opts", A.RenderOpts),
-           ("nrrt_render_stats", A.RenderStats), ("nrrt_camera_file", A.CameraFile), ("nrrt_adaptive_opts", A.AdaptiveOpts)]
+           ("nrrt_render_stats", A.RenderStats), ("nrrt_camera_file", A.CameraFile), ("nrrt_adaptive_opts", A.AdaptiveOpts),
+           ("nrrt_denoise_opts", A.DenoiseOpts)]
 NAMES = {cls: name for name, cls in STRUCTS}
 SCALARS = {C.c_uint32: "u32", C.c_uint64: "u64", C.c_double: "f64", C.c_float: "f32", C.c_uint8: "u8", C.c_int: "c_int"}
 # which = index accepted by nrrt_abi_sizeof (header order, see include/nrrt.h)
 SIZEOF_ORDER = ["nrrt_object", "nrrt_material", "nrrt_texture", "nrrt_image", "nrrt_graph_desc", "nrrt_camera_config",
                 "nrrt_camera", "nrrt_node", "nrrt_box", "nrrt_xform", "nrrt_instance", "nrrt_scene_desc", "nrrt_hit",
                 "nrrt_trace_stats", "nrrt_render_opts", "nrrt_render_stats", "nrrt_camera_file", "nrrt_wnode",
-                "nrrt_hit_compact", "nrrt_adaptive_opts"]
+                "nrrt_hit_compact", "nrrt_adaptive_opts", "nrrt_denoise_opts"]
 
 
 def rust_type(t, field=""):
@@ -151,6 +152,9 @@ extern "C" {
     pub fn nrrt_pass_items_active(width: u32, height: u32, samples_per_pixel: u32, rank: u32, world: u32,
                                   rows_per_block: u32, c0: u32, c1: u32, active: *const u32, n_active: u32, first: u32,
                                   n: u32, out: *mut u32) -> u32;
+    // denoising: first-hit guides of a frame and the a-trous filter on an adaptive frame (an extra output)
+    pub fn nrrt_accum_aov(accum: *mut nrrt_accum, aov_samples: u32, albedo: *mut f32, normal: *mut f32, flags: u32) -> c_int;
+    pub fn nrrt_accum_denoise(accum: *mut nrrt_accum, opts: *const nrrt_denoise_opts, out_rgb: *mut f32, flags: u32) -> c_int;
     pub fn nrrt_abi_sizeof(which: c_int) -> usize;
 }
 '''

@@ -1,6 +1,7 @@
 #!/usr/bin/env python3
 """Small renders for compute-sanitizer (developer tool, GPU box): every kernel design on a 64x36 Cornell box, the
-pooled and fused kernels on the teapot mesh and the sphere field, an adaptive frame in every design, scenes whose
+pooled and fused kernels on the teapot mesh and the sphere field, an adaptive frame in every design, the denoising
+guides and filter (odd sizes: taps past every border), scenes whose
 traversal stacks are full by construction (four instance levels, 65536 instances), a fixed-ray batch each.
   compute-sanitizer --tool memcheck  python tools/sanitize_run.py
   compute-sanitizer --tool racecheck python tools/sanitize_run.py"""
@@ -51,6 +52,19 @@ for m in (A.MODE_FUSED, A.MODE_POOL, A.MODE_WAVEFRONT, A.MODE_MEGAKERNEL):
     ref = (img, n) if ref is None else ref
     assert np.array_equal(img, ref[0]) and np.array_equal(n, ref[1])
     print("adaptive", A.MODE_NAMES[m], "active per pass", passes, "mean samples", float(n.mean()), flush=True)
+# denoising: the guide pass (k_aov, on a partition too) and every filter iteration (k_denoise_*: the checked build
+# bounds-checks each tap) on odd sizes, so that taps fall past every border at every spacing
+for W, H in ((1, 1), (7, 3), (33, 17)):
+    gd = load_scene("scenes/earth.toml", camera_override=CameraConfig(width=W, height=H, samples_per_pixel=6, ray_max_bounces=8))
+    hs = api.HostScene(gd)
+    ctx.upload(hs)
+    cam_d = api.camera_build(gd.camera.to_builder_config())
+    with ctx.progressive(cam_d, seed=1, adaptive={"rel_error": 0.0}) as p:
+        p.render(p.samples_per_pixel)
+        out = p.denoised(iterations=8, aov_samples=3)
+    with ctx.progressive(cam_d, seed=1, world=3, rank=1, rows_per_block=1) as p:
+        p.aov(2)
+    print("denoise", W, H, "finite", bool(np.isfinite(out).all()), flush=True)
 # stacks full by construction (tools/instance_scenes.py): four instance levels at max_stack 32, the LITE pool variant at
 # its per-scene cap (binary stack 24), and 65536 instances (ids past 16 bits in the pooled kernel's chain words)
 for name, g, runs in (("full_stack(32)", S.full_stack(32), ((A.MODE_FUSED, None), (A.MODE_POOL, "0"), (A.MODE_WAVEFRONT, None))),
